@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the rasterizer hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md §8(d) config 2): synthetic 1M-Gaussian
 scene, SH degree 3, one 1920x1080 view per step, rasterizer forward + backward with
@@ -22,6 +22,12 @@ Rank 0 prints ONE JSON line:
 (oracle/_ref/ref_rasterizer_C.so) on the same inputs / metric; the reference has no CPU
 implementation of this path, so its own implementation is timed on the same GPU.  If that
 build is absent the CPU restatement is timed instead (kind "port").
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident leg returned (rank 0) as DIR/<name>.npy
+in float32 (integer outputs as float64): the forward's images and per-Gaussian radii / observe counts, num_rendered,
+and the nine gradient arrays of the backward.  Larger outputs are stored as a fixed sample that depends only on their
+shape (seeded pixel and Gaussian indices, at most DUMP_PIXELS / DUMP_GAUSSIANS of them, about 52 MB in all at the
+default workload), so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -33,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree: it leaves no __pycache__ behind
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -42,6 +49,10 @@ WIDTH = int(os.environ.get("HG_BENCH_W", 1920))
 HEIGHT = int(os.environ.get("HG_BENCH_H", 1080))
 METRIC = "fwd+bwd Mpix/s @1M Gaussians 1080p"
 UNIT = "Mpix/s"
+DUMP_PIXELS = 1 << 18     # sampled pixels of every image output (10 floats each over colour, all_map and depths)
+DUMP_GAUSSIANS = 1 << 17  # sampled Gaussian rows of every per-Gaussian output (78 floats each)
+GRAD_NAMES = ("dL_dmeans2D", "dL_dcolors", "dL_dopacity", "dL_dmeans3D", "dL_dcov3D", "dL_dsh", "dL_dscales",
+              "dL_drotations", "dL_dall_map")  # the order rasterize_gaussians_backward returns them in
 
 
 # ----------------------------------------------------------------------------- helpers
@@ -89,7 +100,8 @@ def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    # no measurement on this machine: the HBM copy bandwidth the project measured on a B200 (BASELINE.md §2)
+    return 6544.0, "BASELINE.md §2 (measured on a B200; power limit not recorded)"
 
 
 def camera_for(rank, step):
@@ -98,6 +110,31 @@ def camera_for(rank, step):
     dx = 0.25 * ((rank * 7 + step * 3) % 5 - 2) if (rank or step) else 0.0
     dy = 0.15 * ((rank * 5 + step) % 3 - 1) if (rank or step) else 0.0
     return syn.default_camera(WIDTH, HEIGHT, eye=(dx, dy, -5.0))
+
+
+def _sample(n, k, seed):
+    """Sorted indices of a fixed seeded sample of k of n elements (all of them when n <= k)."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+
+def dump_outputs(out_dir, fwd, grads):
+    """Write the outputs of one rasterizer forward + backward call (see --dump-outputs) to out_dir/<name>.npy."""
+    R, color, radii, observe, all_map, plane_depth, geom, binning, img, invdepth = fwd
+    os.makedirs(out_dir, exist_ok=True)
+    pix = torch.from_numpy(_sample(color.shape[1] * color.shape[2], DUMP_PIXELS, seed=1)).to(color.device)
+    rows = torch.from_numpy(_sample(radii.shape[0], DUMP_GAUSSIANS, seed=2)).to(radii.device)
+    out = {"num_rendered": np.array([R], np.float64)}
+    for name, t in (("color", color), ("all_map", all_map), ("plane_depth", plane_depth), ("invdepth", invdepth)):
+        out[name] = t.reshape(t.shape[0], -1).index_select(1, pix).float().cpu().numpy()
+    for name, t in (("radii", radii), ("out_observe", observe)):
+        out[name] = t.index_select(0, rows).cpu().numpy().astype(np.float64)
+    for name, t in zip(GRAD_NAMES, grads):
+        if t is not None:  # dL_dsh is None where the backward writes SH factors for a multi-GPU exchange instead
+            out[name] = t.index_select(0, rows).float().cpu().numpy()
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def stage_bytes(N, Nv, R, HW, T):
@@ -307,12 +344,13 @@ def run_gpu_arm(args, impl):
             grads = C.rasterize_gaussians_backward(*bwd_tuple(fa, fwd, g), **kw)
             if ddp:
                 pack_and_allreduce(grads)
-        return fwd
+        # only the last timed step's gradients outlive the call (for --dump-outputs)
+        return fwd, (grads if s == Wm + K - 1 else None)
 
     for c in cams:
         c.to(dev)
     for s in range(Wm):
-        fwd = step_resident(s)
+        fwd, grads = step_resident(s)
     torch.cuda.synchronize()
     if ddp:
         dist.barrier()
@@ -326,7 +364,7 @@ def run_gpu_arm(args, impl):
     torch.cuda.synchronize()
     e0.record()
     for s in range(Wm, Wm + K):
-        fwd = step_resident(s)
+        fwd, grads = step_resident(s)
     e1.record()
     torch.cuda.synchronize()
     if ddp:
@@ -338,6 +376,9 @@ def run_gpu_arm(args, impl):
         _lib.profile_enable(False)
         stages = _lib.profile_collect()
         launches = int(_lib.lib().hg_launch_count())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fwd, grads)
+    del grads
     R = int(fwd[0])
     Nv = int((fwd[2] > 0).sum())
     t_ms = torch.tensor([ms_total], device=dev)
@@ -473,26 +514,26 @@ def run_gpu_arm(args, impl):
         del params, am_param, scene, all_maps
         torch.cuda.empty_cache()
         n_train = int(os.environ.get("HG_BENCH_TRAIN_N", 2_000_000))
-        train = train_leg(dev, rank, world, ddp, steps=max(2, min(K, 5)), warmup=3, views_per_rank=8, n_gauss=n_train,
+        train = train_leg(dev, rank, world, ddp, steps=K, warmup=3, views_per_rank=8, n_gauss=n_train,
                           recipe="uav")
         torch.cuda.empty_cache()
         # the same step with every ground-truth-only quantity recomputed at every visit (SURVEY.md §8(d): both)
-        unc_uav = train_leg(dev, rank, world, ddp, steps=max(2, min(K, 5)), warmup=3, views_per_rank=8, n_gauss=n_train,
+        unc_uav = train_leg(dev, rank, world, ddp, steps=K, warmup=3, views_per_rank=8, n_gauss=n_train,
                             recipe="uav", cache_gt=False)
         train["views_per_s_uncached_ground_truth"] = unc_uav["views_per_s"]
         train["ms_per_step_uncached_ground_truth"] = unc_uav["ms_per_step"]
         if world == 1:
             torch.cuda.empty_cache()
-            train_c3 = train_leg(dev, rank, world, False, steps=max(3, min(K, 10)), warmup=3, views_per_rank=1,
+            train_c3 = train_leg(dev, rank, world, False, steps=K, warmup=3, views_per_rank=1,
                                  n_gauss=n_train, recipe="c2")
             torch.cuda.empty_cache()
             # the same step with every ground-truth-only quantity recomputed at every visit (no per-camera cache)
-            unc = train_leg(dev, rank, world, False, steps=max(3, min(K, 10)), warmup=3, views_per_rank=1,
+            unc = train_leg(dev, rank, world, False, steps=K, warmup=3, views_per_rank=1,
                             n_gauss=n_train, recipe="c2", cache_gt=False)
             train_c3["views_per_s_uncached_ground_truth"] = unc["views_per_s"]
             sys.path.insert(0, os.path.join(ROOT, "tools"))
             import loss_bench
-            losses = loss_bench.measure(dev, iters=10, warmup=3, cpu=not os.environ.get("HG_BENCH_SKIP_CPU"))
+            losses = loss_bench.measure(dev, iters=K, warmup=3, cpu=not os.environ.get("HG_BENCH_SKIP_CPU"))
 
     if rank != 0:
         if ddp:
@@ -847,6 +888,8 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", 0))
@@ -856,6 +899,8 @@ def main():
             return
         if have_ref and torch.cuda.is_available():
             run_gpu_arm(args, "reference")
+        elif args.dump_outputs:
+            raise SystemExit("--dump-outputs needs the GPU arm: the CPU restatement is timed here, not the device path")
         else:
             run_cpu_reference(args)
         return
