@@ -7,7 +7,8 @@ EXPORTED_SYMBOLS = (
     "hg_geometry_all_map", "hg_geometry_all_map_backward", "hg_activate_params", "hg_activate_params_backward", "hg_prologue_backward", "hg_depth_normal", "hg_depth_normal_backward",
     "hg_normal_consistency_workspace_bytes", "hg_normal_consistency_loss", "hg_adam_step", "hg_densification_stats", "hg_expand_to_size_workspace_bytes", "hg_expand_to_size",
     "hg_interpolation_weights", "hg_hier_interpolate", "hg_hier_interpolate_backward",
-    "hg_dist2_knn3_workspace_bytes", "hg_dist2_knn3",
+    "hg_dist2_knn3_workspace_bytes", "hg_dist2_knn3", "hg_densify_workspace_bytes", "hg_densify_plan", "hg_densify_apply",
+    "hg_reset_opacity",
 )
 
 
@@ -26,6 +27,7 @@ def lib():
         return L
     vp, i32, i64, sz, f32, ci = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_size_t, ctypes.c_float, ctypes.c_int
     f64 = ctypes.c_double
+    p64 = ctypes.POINTER(i64)
     proto = {
         "hg_geometry_all_map": (ci, [vp, vp, vp, vp, vp, i64, vp, vp]),
         "hg_geometry_all_map_backward": (ci, [vp, vp, vp, vp, vp, i64, vp, vp, vp, vp]),
@@ -46,6 +48,10 @@ def lib():
         "hg_hier_interpolate_backward": (ci, [vp, i64, i32, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
         "hg_dist2_knn3_workspace_bytes": (sz, [i64]),
         "hg_dist2_knn3": (ci, [vp, i64, vp, vp, vp]),
+        "hg_densify_workspace_bytes": (sz, [i64]),
+        "hg_densify_plan": (ci, [vp, p64, i64, vp, i32, f64, f64, f64, f64, f64, vp, p64, p64, p64, p64, vp]),
+        "hg_densify_apply": (ci, [vp, vp, vp, p64, i64, vp, vp, vp, p64, i64, vp, ctypes.c_uint64, vp, vp]),
+        "hg_reset_opacity": (ci, [vp, vp, vp, i64, vp]),
     }
     for name, (res, args) in proto.items():
         fn = getattr(L, name)

@@ -19,6 +19,7 @@ of culled Gaussians unwritten (HG_BWD_SKIP_CULLED_ROWS) and ONE kernel (`hg_prol
 from the rasterizer's gradients to the raw-parameter arena (all_map backward, scale-regulariser gradient, activation
 chain rule, accumulation); the activations themselves are computed once per optimiser step.
 """
+import ctypes
 import math
 
 import torch
@@ -55,6 +56,17 @@ class OptimizationParams:
     lambda_freq = 0.001
     lambda_scale = 0.005
     freq_warmup_iterations = 1000
+    # adaptive density control (ViewShardedTrainer(densify=True)); intervals count optimiser steps.  The reference ships
+    # no train.py, so these are not read from it: intervals, percent_dense and min_opacity are graphdeco 3DGS's
+    # (arguments/__init__.py, train.py), the gradient threshold is hierarchical-3DGS's, whose statistic is the same
+    # running maximum of the screen-space gradient norm this build accumulates (not a mean)
+    densify_from_iter = 500
+    densify_until_iter = 15_000
+    densification_interval = 100
+    opacity_reset_interval = 3000
+    densify_grad_threshold = 0.015
+    percent_dense = 0.01
+    min_opacity = 0.005
 
 
 class _ActivateParams(torch.autograd.Function):
@@ -131,6 +143,69 @@ def morton_order(xyz):
     return torch.argsort(code, stable=True)
 
 
+def arena_layout(N):
+    """({group: first float}, total floats) of the parameter / gradient / moment arenas of N Gaussians: the GROUPS in
+    order, every group starting on a multiple of 4 floats (16 bytes) — the fused kernels move rotation / feature rows
+    as float4 and the in-fabric exchange works on 16-byte units, for ANY Gaussian count (pad floats stay zero)."""
+    starts, total = {}, 0
+    for name, w in GROUPS:
+        starts[name] = total
+        total += (N * w + 3) // 4 * 4
+    return starts, total
+
+
+def densify_arenas(param_arena, exp_avg, exp_avg_sq, N, accum, max_grad, min_opacity, extent, max_screen_size=None,
+                   seed=0, samples=None, percent_dense=0.01, skybox_points=0):
+    """graphdeco 3DGS densify_and_clone + densify_and_split + prune over flat arenas of N rows (arena_layout; DESIGN.md
+    §3 "Densify and prune"): returns (new parameter arena, new exp_avg, new exp_avg_sq, counts) with counts =
+    dict(kept, cloned, split, pruned, n): original rows kept, rows cloned, rows split, rows pruned (originals, clones
+    and children), n = N'.  `accum` [N] fp32: the max-form screen-space gradient
+    statistic.  Children are drawn from Philox4x32-10 keyed by `seed` (the same bits on every rank), or taken from
+    `samples` [2 |split|, 3] (torch.normal(0, stds.repeat(2, 1)) of the reference).  One host synchronisation.
+    Raises ValueError when nothing would be left (N' = 0)."""
+    dev = param_arena.device
+    L = _G()
+    st = torch.cuda.current_stream(dev).cuda_stream
+    ws = torch.empty(int(L.hg_densify_workspace_bytes(N)), dtype=torch.uint8, device=dev)
+    starts, _total = arena_layout(N)
+    off = (ctypes.c_int64 * 5)(*[starts[n] for n, _ in GROUPS])
+    kept, cloned, split, new_n = (ctypes.c_int64() for _ in range(4))
+    accum = accum.contiguous()
+    with torch.cuda.device(dev):
+        rc = L.hg_densify_plan(param_arena.data_ptr(), off, N, accum.data_ptr(), int(skybox_points), float(max_grad),
+                               float(min_opacity), float(extent), float(max_screen_size or 0.0), float(percent_dense),
+                               ws.data_ptr(), ctypes.byref(kept), ctypes.byref(cloned), ctypes.byref(split),
+                               ctypes.byref(new_n), st)
+    _lib.check(rc, "densify_plan")
+    n2 = new_n.value
+    counts = dict(kept=kept.value, cloned=cloned.value, split=split.value, pruned=N + cloned.value + split.value - n2,
+                  n=n2)
+    if n2 == 0:
+        raise ValueError("densify_and_prune would leave no Gaussians (%s)" % counts)
+    starts2, total2 = arena_layout(n2)
+    off2 = (ctypes.c_int64 * 5)(*[starts2[n] for n, _ in GROUPS])
+    # every float of the new arenas (pads included) is written by the kernel
+    new = [torch.empty(total2, dtype=torch.float32, device=dev) for _ in range(3)]
+    if samples is not None:
+        samples = samples.to(device=dev, dtype=torch.float32).contiguous()
+        if tuple(samples.shape) != (2 * split.value, 3):
+            raise ValueError("samples must be [2 * %d, 3], got %s" % (split.value, tuple(samples.shape)))
+    with torch.cuda.device(dev):
+        rc = L.hg_densify_apply(param_arena.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), off, N,
+                                new[0].data_ptr(), new[1].data_ptr(), new[2].data_ptr(), off2, n2,
+                                samples.data_ptr() if samples is not None and samples.numel() else None,
+                                int(seed) & 0xFFFFFFFFFFFFFFFF, ws.data_ptr(), st)
+    _lib.check(rc, "densify_apply")
+    return new[0], new[1], new[2], counts
+
+
+def cameras_extent(cameras):
+    """Scene extent of the densification thresholds: 1.1 x the largest distance of a camera centre from their mean
+    (the radius of the reference's getNerfppNorm)."""
+    c = torch.stack([torch.as_tensor(cam.camera_center, dtype=torch.float64).reshape(3).cpu() for cam in cameras])
+    return float(torch.linalg.norm(c - c.mean(0), dim=1).max()) * 1.1
+
+
 class GaussianParams:
     """Trainable Gaussians in the reference's parameterisation (scene/gaussian_model.py:60-140): raw leaves
     `_xyz`, `_features` (N,16,3), `_opacity` (logit), `_scaling` (log), `_rotation` (un-normalised quaternion) and the
@@ -138,16 +213,31 @@ class GaussianParams:
     into one flat gradient arena of the same layout."""
 
     def __init__(self, xyz, features, opacity_logit, scaling_log, rotation, sh_degree=3):
-        dev = xyz.device
         N = xyz.size(0)
-        self.N = N
-        # every group starts on a multiple of 4 floats (16 bytes): the fused kernels move rotation / feature rows as
-        # float4 and the in-fabric exchange works on 16-byte units, for ANY Gaussian count (pad floats stay zero)
-        starts, total = {}, 0
+        starts, total = arena_layout(N)
+        param_arena = torch.zeros(total, dtype=torch.float32, device=xyz.device)
+        src = dict(xyz=xyz, features=features.reshape(N, -1), opacity=opacity_logit, scaling=scaling_log, rotation=rotation)
         for name, w in GROUPS:
-            starts[name] = total
-            total += (N * w + 3) // 4 * 4
-        self.param_arena = torch.zeros(total, dtype=torch.float32, device=dev)
+            param_arena[starts[name]:starts[name] + N * w].view(N, w).copy_(src[name].reshape(N, w))
+        self._attach(param_arena, N)
+        self.active_sh_degree = self.max_sh_degree = sh_degree
+        self.skybox_points = 0
+        self.order = None
+        # fused activations (CUDA only): one kernel per view forward, one backward that also accumulates into the arena
+        self.fused = xyz.is_cuda
+        self._act = None          # (xyz, features, opacity, scaling, rotation) of the current view
+        self._grad_dirty = False  # False: the next fused backward overwrites the arena (no zero fill needed)
+        self.sh_sink = self.fused  # SH gradient accumulated by the rasterizer's own backward kernel
+        self._sink_used = False
+
+    def _attach(self, param_arena, N):
+        """Adopt `param_arena` (arena_layout(N)) with a fresh gradient arena of the same layout, the leaves and their
+        `.grad` views.  The constructor and `resize` both come through here.  Where the gradient arena is multicast
+        symmetric memory its allocation is collective: every rank calls this with the same N."""
+        dev = param_arena.device
+        starts, total = arena_layout(N)
+        self.N = N
+        self.param_arena = param_arena
         # the gradient arena is born where the per-step exchange wants it: multicast symmetric memory when the ranks
         # share an NVSwitch (in-fabric all-reduce kernel), a plain tensor otherwise (NCCL / gloo all-reduce)
         self.exchange = None
@@ -155,26 +245,24 @@ class GaussianParams:
             self.grad_arena, self.exchange = parallel.make_exchange_arena(total, dev)
         else:
             self.grad_arena = torch.zeros(total, dtype=torch.float32, device=dev)
-        src = dict(xyz=xyz, features=features.reshape(N, -1), opacity=opacity_logit, scaling=scaling_log, rotation=rotation)
         self.leaves, self.slices = {}, {}
         for name, w in GROUPS:
-            off = starts[name]
-            sl = slice(off, off + N * w)
+            sl = slice(starts[name], starts[name] + N * w)
             self.slices[name] = sl
-            self.param_arena[sl].view(N, w).copy_(src[name].reshape(N, w))
             shape = (N, 16, 3) if name == "features" else (N, w)
             leaf = self.param_arena[sl].view(shape).requires_grad_(True)
             leaf.grad = self.grad_arena[sl].view(shape)
             self.leaves[name] = leaf
         self._xyz, self._features = self.leaves["xyz"], self.leaves["features"]
         self._opacity, self._scaling, self._rotation = self.leaves["opacity"], self.leaves["scaling"], self.leaves["rotation"]
-        self.active_sh_degree = self.max_sh_degree = sh_degree
-        self.skybox_points = 0
-        # fused activations (CUDA only): one kernel per view forward, one backward that also accumulates into the arena
-        self.fused = xyz.is_cuda
-        self._act = None          # (xyz, features, opacity, scaling, rotation) of the current view
-        self._grad_dirty = False  # False: the next fused backward overwrites the arena (no zero fill needed)
-        self.sh_sink = self.fused  # SH gradient accumulated by the rasterizer's own backward kernel
+
+    def resize(self, param_arena, N):
+        """Adopt a parameter arena of N rows (densify_and_prune): new gradient arena, leaves and `.grad` views.  The
+        rows are no longer along the Morton curve of `from_scene(spatial_order=True)`: `.order` becomes None."""
+        self._attach(param_arena, N)
+        self.order = None
+        self._act = None
+        self._grad_dirty = False
         self._sink_used = False
 
     @classmethod
@@ -240,6 +328,11 @@ class ArenaAdam:
         self.lr = dict(xyz=opt.position_lr_init * spatial_lr_scale, features=opt.feature_lr, opacity=opt.opacity_lr,
                        scaling=opt.scaling_lr, rotation=opt.rotation_lr)
         self.eps, self.step_count = eps, 0
+
+    def resize(self, exp_avg, exp_avg_sq):
+        """Adopt moment arenas of the parameters' new size (densify_and_prune); the step count carries on, as
+        cat_tensors_to_optimizer keeps state["step"]."""
+        self.exp_avg, self.exp_avg_sq = exp_avg, exp_avg_sq
 
     @torch.no_grad()
     def step(self, grad_scale=1.0, visible_mask=None):
@@ -319,8 +412,16 @@ def balance_views(costs, world, speeds=None):
 
 class ViewShardedTrainer:
     def __init__(self, params: GaussianParams, background, opt=OptimizationParams, pipe=PipelineParams, group=None,
-                 sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0):
+                 sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0, densify=False,
+                 scene_extent=None):
+        """`densify`: run the adaptive density control schedule of the OptimizationParams densify_* fields inside
+        `step()` (off by default); it needs `scene_extent` (`cameras_extent(cameras)`) and turns the densification
+        statistics on."""
         self.params, self.bg, self.opt, self.pipe, self.group = params, background, opt, pipe, group
+        if densify and scene_extent is None:
+            raise ValueError("densify=True needs scene_extent (cameras_extent(cameras))")
+        self.densify, self.scene_extent = densify, scene_extent
+        densification_stats = densification_stats or densify
         self.adam = ArenaAdam(params, opt)
         # the reference steps its optimiser on the rows that were visible (`optimizer.step(relevant)`, OurAdam.py:106)
         self.sparse_adam = sparse_adam and params.param_arena.is_cuda
@@ -331,10 +432,8 @@ class ViewShardedTrainer:
         self._gt_cache = {}
         self.densification_stats = densification_stats and params.param_arena.is_cuda
         if self.densification_stats:  # GaussianModel.training_setup (scene/gaussian_model.py:282-294)
-            dev = params.param_arena.device
-            self.xyz_gradient_accum = torch.zeros((params.N, 1), device=dev)
-            self.denom = torch.zeros((params.N, 1), device=dev)
-            self.max_radii2D = torch.zeros(params.N, device=dev)
+            self._zero_densification_stats()
+        self._opacity_resets = 0
         # the frequency / scale regulariser switches on at opt.freq_warmup_iterations, as the reference's
         # frequency_regularization_pyramid_scale(iteration, warmup_iterations=1000) does; `start_iteration` resumes a run
         self.iteration = int(start_iteration)
@@ -588,10 +687,70 @@ class ViewShardedTrainer:
                 dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=self.group)
                 n_views = int(round(float(cnt.item())))
         self.adam.step(grad_scale=1.0 / max(n_views, 1), visible_mask=self.visible if self.sparse_adam else None)
+        if getattr(self, "densify", False):
+            self._density_schedule()
         if timing is not None:
             ev[2].record()
             timing.append(ev)
         return total
+
+    def _zero_densification_stats(self):
+        dev, N = self.params.param_arena.device, self.params.N
+        self.xyz_gradient_accum = torch.zeros((N, 1), device=dev)
+        self.denom = torch.zeros((N, 1), device=dev)
+        self.max_radii2D = torch.zeros(N, device=dev)
+
+    @torch.no_grad()
+    def densify_and_prune(self, max_grad, min_opacity, extent, max_screen_size=None, seed=None):
+        """GaussianModel.densify_and_prune of graphdeco 3DGS over the arenas (DESIGN.md §3 "Densify and prune"): clone
+        the small Gaussians whose gradient statistic reaches `max_grad`, split the large ones in two, prune the
+        transparent ones (and, with `max_screen_size`, the ones larger than 0.1 `extent` in world space).  With several
+        ranks the statistics are combined first (gradient and radius by MAX, visit count by SUM), so every rank makes
+        the same decisions and draws the same children: the arenas stay bit-identical.  `seed` keys the split draws
+        (default: the iteration).  Returns the counts of `densify_arenas` (cloned, split, pruned, n = N', ...); raises ValueError, leaving the model as
+        it was, if no Gaussian would be left."""
+        if not self.densification_stats:
+            raise RuntimeError("densify_and_prune needs ViewShardedTrainer(densification_stats=True)")
+        p = self.params
+        if self.world > 1:
+            dist.all_reduce(self.xyz_gradient_accum, op=dist.ReduceOp.MAX, group=self.group)
+            dist.all_reduce(self.max_radii2D, op=dist.ReduceOp.MAX, group=self.group)
+            dist.all_reduce(self.denom, op=dist.ReduceOp.SUM, group=self.group)
+        new_p, new_m, new_v, counts = densify_arenas(
+            p.param_arena, self.adam.exp_avg, self.adam.exp_avg_sq, p.N, self.xyz_gradient_accum.view(-1), max_grad,
+            min_opacity, extent, max_screen_size, self.iteration if seed is None else seed,
+            percent_dense=getattr(self.opt, "percent_dense", 0.01), skybox_points=p.skybox_points)
+        p.resize(new_p, counts["n"])
+        self.adam.resize(new_m, new_v)
+        self.visible = torch.zeros(p.N, dtype=torch.uint8, device=new_p.device)
+        self._zero_densification_stats()
+        self._step_activations = None
+        return counts
+
+    @torch.no_grad()
+    def reset_opacity(self):
+        """GaussianModel.reset_opacity: opacity = min(opacity, 0.01) (through the logit), with that group's Adam moments
+        zeroed (replace_tensor_to_optimizer); every other float of the arenas is left as it is."""
+        p = self.params
+        sl = p.slices["opacity"]
+        with torch.cuda.device(p.param_arena.device):
+            rc = _G().hg_reset_opacity(p.param_arena[sl].data_ptr(), self.adam.exp_avg[sl].data_ptr(),
+                                       self.adam.exp_avg_sq[sl].data_ptr(), p.N, torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "reset_opacity")
+        p._act = None
+
+    def _density_schedule(self):
+        """graphdeco's train.py schedule, after the optimiser step of step `it`: densify every densification_interval
+        steps in (densify_from_iter, densify_until_iter), with the size threshold 20 once the opacity has been reset;
+        reset the opacity every opacity_reset_interval steps before densify_until_iter."""
+        o, it = self.opt, self.iteration
+        if it >= o.densify_until_iter:
+            return
+        if it > o.densify_from_iter and it % o.densification_interval == 0:
+            self.densify_and_prune(o.densify_grad_threshold, o.min_opacity, self.scene_extent,
+                                   20 if it > o.opacity_reset_interval else None)
+        if it % o.opacity_reset_interval == 0:
+            self.reset_opacity()
 
     def _add_densification_stats(self, pkg):
         g = pkg["means2D_grad"] if "means2D_grad" in pkg else pkg["viewspace_points"].grad

@@ -132,6 +132,35 @@ HG_API int hg_adam_step(float *param, const float *grad, float *exp_avg, float *
 HG_API int hg_densification_stats(const float *grad_means2D, const int32_t *radii, int64_t N,
                                   float *xyz_gradient_accum, float *denom, float *max_radii2D, void *stream);
 
+/* Adaptive density control over the training arenas (DESIGN.md §3 "Densify and prune"): graphdeco 3DGS
+ * densify_and_clone + densify_and_split + prune, in three steps.  An arena holds the five groups of N rows
+ * xyz 3 | features 48 | opacity 1 (logit) | scaling 3 (log) | rotation 4, each starting at group_offsets[g] (host
+ * int64 [5], in floats, multiples of 4; GaussianParams' layout), 16-byte aligned.
+ *   hg_densify_plan: g = accum (NaN -> 0), smax = max exp(scaling); clone C = |g| >= max_grad && smax <= (float)(
+ *     percent_dense * extent); split S = g >= max_grad && smax > that; a row of the output is pruned when
+ *     sigmoid(opacity) < min_opacity or (max_screen_size > 0, 0 = None) smax > (float)(0.1 * extent).  Writes the
+ *     decisions into `workspace` (hg_densify_workspace_bytes(N) bytes) and returns through host out-params the kept
+ *     original rows, |C|, |S| and N'.  Synchronises the stream once (N' sizes the new arenas).  A model with
+ *     skybox_points != 0 is rejected.
+ *   hg_densify_apply: from the same workspace, writes the N' rows [kept rows | clones | first children | second
+ *     children] (each in source order, pruned rows left out) into the new parameter arena and both new Adam moment
+ *     arenas (kept rows keep their moments, new rows start at zero; pad floats are zeroed).  Children: xyz = R(q) s + xyz
+ *     with s = exp(scaling) * z, z ~ N(0, I) from Philox4x32-10 (key = seed, counter = (source row, child)), or
+ *     s = samples [2|S|, 3] (rows: first children, then second children, in source order) when non-NULL;
+ *     scaling = log(exp(scaling) / 1.6); features, opacity, rotation copied.
+ *   hg_reset_opacity: opacity = inverse_sigmoid(min(sigmoid(opacity), 0.01)) over N floats, and that group's two
+ *     moment blocks zeroed. */
+HG_API size_t hg_densify_workspace_bytes(int64_t N);
+HG_API int hg_densify_plan(const float *param, const int64_t *group_offsets, int64_t N, const float *accum,
+                           int32_t skybox_points, double max_grad, double min_opacity, double extent,
+                           double max_screen_size, double percent_dense, void *workspace, int64_t *out_kept,
+                           int64_t *out_cloned, int64_t *out_split, int64_t *out_new_n, void *stream);
+HG_API int hg_densify_apply(const float *old_param, const float *old_exp_avg, const float *old_exp_avg_sq,
+                            const int64_t *old_offsets, int64_t N, float *new_param, float *new_exp_avg,
+                            float *new_exp_avg_sq, const int64_t *new_offsets, int64_t new_n, const float *samples,
+                            uint64_t seed, const void *workspace, void *stream);
+HG_API int hg_reset_opacity(float *opacity, float *exp_avg, float *exp_avg_sq, int64_t N, void *stream);
+
 /* Hierarchy LOD cut (SURVEY.md §8(f) f1).  nodes [N,7] i32 (types.h:47-56: depth, parent, start, count_leafs,
  * count_merged, start_children, count_children), boxes [N,2,4] f32 (min xyz + extent, max xyz + pad), viewpoint [3] on
  * the device.  hg_expand_to_size = Switching::expandToSize (runtime_switching.cu:496-527): for every node whose
