@@ -6,6 +6,7 @@ parameter tensor through hg_adam_step (include/hidegs_geometry.h), without the g
     opt = Adam([{"params": [xyz], "lr": 1.6e-4, "name": "xyz"}, ...], lr=0.0, eps=1e-15)
     opt.step(relevant)      # relevant: empty tensor (all rows), int64 index tensor, or bool mask over the rows
 """
+import numpy as np
 import torch
 
 from . import _lib
@@ -56,3 +57,20 @@ class Adam(torch.optim.Optimizer):
                         float(group["eps"]), int(state["step"]), float(grad_scale), 0, 0.0, torch.cuda.current_stream().cuda_stream)
                 _lib.check(rc, "adam_step")
         return loss
+
+
+def get_expon_lr_func(lr_init, lr_final, lr_delay_steps=0, lr_delay_mult=1.0, max_steps=1000000):
+    """graphdeco 3DGS's learning-rate schedule (utils/general_utils.py get_expon_lr_func): log-linear from lr_init at
+    step 0 to lr_final at max_steps (held there after), times a delay factor that rises from lr_delay_mult to 1 along a
+    quarter sine over the first lr_delay_steps steps.  A negative step, or lr_init = lr_final = 0, gives 0."""
+    def helper(step):
+        if step < 0 or (lr_init == 0.0 and lr_final == 0.0):
+            return 0.0
+        if lr_delay_steps > 0:
+            delay_rate = lr_delay_mult + (1 - lr_delay_mult) * np.sin(0.5 * np.pi * np.clip(step / lr_delay_steps, 0, 1))
+        else:
+            delay_rate = 1.0
+        t = np.clip(step / max_steps, 0, 1)
+        log_lerp = np.exp(np.log(lr_init) * (1 - t) + np.log(lr_final) * t)
+        return float(delay_rate * log_lerp)
+    return helper

@@ -67,6 +67,15 @@ class OptimizationParams:
     densify_grad_threshold = 0.015
     percent_dense = 0.01
     min_opacity = 0.005
+    # per-image exposure (ViewShardedTrainer(train_exposure=True)): Adam with eps 1e-8 over the whole table, lr
+    # get_expon_lr_func(exposure_lr_init, exposure_lr_final, exposure_lr_delay_steps, exposure_lr_delay_mult,
+    # max_steps=iterations) at the trainer's iteration.  The reference ships no train.py; these are hierarchical-3DGS's
+    # arguments/__init__.py values as recalled, not read from or checked against a reference tree
+    exposure_lr_init = 0.01
+    exposure_lr_final = 0.0001
+    exposure_lr_delay_steps = 5000
+    exposure_lr_delay_mult = 0.001
+    iterations = 30_000
 
 
 class _ActivateParams(torch.autograd.Function):
@@ -229,6 +238,50 @@ class GaussianParams:
         self._grad_dirty = False  # False: the next fused backward overwrites the arena (no zero fill needed)
         self.sh_sink = self.fused  # SH gradient accumulated by the rasterizer's own backward kernel
         self._sink_used = False
+        self.exposure_mapping = None  # per-image exposure: setup_exposures
+        self._exposure = self.exposure_grad = None
+
+    def setup_exposures(self, image_names, exposures=None):
+        """Per-image exposure table of the reference's GaussianModel (`_exposure`, `exposure_mapping`; applied by
+        render(..., use_trained_exp=True), DESIGN.md §3 "Per-image exposure"): row i is the [3, 4] affine of
+        image_names[i], eye(3, 4) to start with, or exposures[name] (a load_exposures dict, which must cover every
+        name).  The leaf `_exposure` [n, 3, 4] has its `.grad` aliasing `exposure_grad`, as the arena leaves alias the
+        gradient arena.  The table is per image, not per Gaussian: densify_and_prune and resize leave it alone."""
+        names = list(image_names)
+        if len(set(names)) != len(names):
+            raise ValueError("setup_exposures: duplicate image names")
+        dev = self.param_arena.device
+        table = torch.eye(3, 4, dtype=torch.float32).repeat(len(names), 1, 1)
+        if exposures is not None:
+            missing = [n for n in names if n not in exposures]
+            if missing:
+                raise ValueError("setup_exposures: no exposure for %s" % missing[:5])
+            for i, n in enumerate(names):
+                table[i] = torch.as_tensor(exposures[n], dtype=torch.float32).cpu().reshape(3, 4)
+        self.exposure_mapping = {n: i for i, n in enumerate(names)}
+        self._exposure = table.to(dev).requires_grad_(True)
+        self.exposure_grad = torch.zeros_like(self._exposure, requires_grad=False)
+        self._exposure.grad = self.exposure_grad
+
+    def exposure_index(self, image_name):
+        """Row of `image_name` in the exposure table; ValueError if there is no table or no such image."""
+        if self.exposure_mapping is None:
+            raise ValueError("no exposure table: call setup_exposures(image_names) first")
+        try:
+            return self.exposure_mapping[image_name]
+        except KeyError:
+            raise ValueError("no exposure for image %r" % (image_name,)) from None
+
+    def get_exposure_from_name(self, image_name):
+        """GaussianModel.get_exposure_from_name: the [3, 4] exposure of `image_name` (a differentiable view of the
+        table), as render(..., use_trained_exp=True) reads it."""
+        return self._exposure[self.exposure_index(image_name)]
+
+    def save_exposures(self, path):
+        """exposure.json of the table (ply_io.save_exposures, rows in mapping order)."""
+        from . import ply_io
+        names = sorted(self.exposure_mapping, key=self.exposure_mapping.get)
+        ply_io.save_exposures(path, self._exposure, names)
 
     def _attach(self, param_arena, N):
         """Adopt `param_arena` (arena_layout(N)) with a fresh gradient arena of the same layout, the leaves and their
@@ -411,15 +464,34 @@ def balance_views(costs, world, speeds=None):
 
 
 class ViewShardedTrainer:
+    train_exposure = False  # (class default: also read by trainers assembled without __init__)
+
     def __init__(self, params: GaussianParams, background, opt=OptimizationParams, pipe=PipelineParams, group=None,
                  sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0, densify=False,
-                 scene_extent=None):
+                 scene_extent=None, train_exposure=False):
         """`densify`: run the adaptive density control schedule of the OptimizationParams densify_* fields inside
         `step()` (off by default); it needs `scene_extent` (`cameras_extent(cameras)`) and turns the densification
-        statistics on."""
+        statistics on.
+        `train_exposure`: render every view through the exposure of its `cam.image_name` and learn the table (off by
+        default); it needs `params.setup_exposures(image_names)` first.  Every step zeroes the exposure gradient table,
+        sums it over the ranks and steps it with its own Adam (eps 1e-8, dense over the whole table, the lr schedule of
+        the OptimizationParams exposure_* fields)."""
         self.params, self.bg, self.opt, self.pipe, self.group = params, background, opt, pipe, group
         if densify and scene_extent is None:
             raise ValueError("densify=True needs scene_extent (cameras_extent(cameras))")
+        self.train_exposure = bool(train_exposure)
+        if self.train_exposure:
+            if params._exposure is None:
+                raise ValueError("train_exposure=True needs params.setup_exposures(image_names)")
+            if not params.fused:
+                raise ValueError("train_exposure=True needs CUDA parameters")
+            from .optim import get_expon_lr_func
+            self.exposure_lr = get_expon_lr_func(opt.exposure_lr_init, opt.exposure_lr_final, opt.exposure_lr_delay_steps,
+                                                 opt.exposure_lr_delay_mult, max_steps=opt.iterations)
+            self.exposure_exp_avg = torch.zeros_like(params._exposure, requires_grad=False)
+            self.exposure_exp_avg_sq = torch.zeros_like(params._exposure, requires_grad=False)
+            self.exposure_step_count = 0
+            self._exposure_ws = None
         self.densify, self.scene_extent = densify, scene_extent
         densification_stats = densification_stats or densify
         self.adam = ArenaAdam(params, opt)
@@ -449,7 +521,11 @@ class ViewShardedTrainer:
         the image (an upload running on a copy stream while the view renders)."""
         o = self.opt
         self.params.begin_view()
-        pkg = gr._render_impl(cam, self.params, self.pipe, self.bg, _visibility_as_mask=self.params.param_arena.is_cuda)
+        exp = self.train_exposure
+        if exp:
+            self.params.exposure_index(cam.image_name)  # (ValueError before any work for an unknown image)
+        pkg = gr._render_impl(cam, self.params, self.pipe, self.bg, use_trained_exp=exp,
+                              _visibility_as_mask=self.params.param_arena.is_cuda)
         if gt_ready is not None:
             torch.cuda.current_stream().wait_event(gt_ready)
         image = pkg["render"]
@@ -496,9 +572,13 @@ class ViewShardedTrainer:
     def view_step_direct(self, cam, gt, iteration, gt_ready=None):
         """Forward AND backward of one view (gradients accumulated into the arena), without autograd.  Returns
         (loss value tensor, dict with "visibility_filter" (mask), "radii", "means2D_grad" — defined on the rendered rows
-        only: the rasterizer's backward does not write the rows of culled Gaussians here)."""
+        only: the rasterizer's backward does not write the rows of culled Gaussians here); with train_exposure also
+        "render", the exposed, clamped image the losses saw."""
         o, p, T = self.opt, self.params, self._Tape
         dev = p.param_arena.device
+        exp_off = None  # byte offset of this camera's exposure row in the table / its gradient table
+        if self.train_exposure:
+            exp_off = 48 * p.exposure_index(cam.image_name)
         with torch.no_grad():
             # ---- forward
             # the activated parameters are the same for every view of one optimiser step: step() keeps them
@@ -519,7 +599,14 @@ class ViewShardedTrainer:
             tR = T(True, True, True, False, True, True, True, False, True, False)
             color, radii, _observe, out_all_map, plane_depth, _inv = _RasterizeGaussians.forward(
                 tR, xyz, xyz, feat, e_f, opacity, scaling, rotation, e_f, all_map_in, rs)
-            image = color.clamp(0, 1)
+            if exp_off is None:
+                image = color.clamp(0, 1)
+            else:  # clamp(color through the camera's exposure, 0, 1): hg_exposure_apply
+                image = torch.empty_like(color)
+                with torch.cuda.device(dev):
+                    rc = lu._L().hg_exposure_apply(color.data_ptr(), p._exposure.data_ptr() + exp_off, color.size(1),
+                                                   color.size(2), image.data_ptr(), torch.cuda.current_stream().cuda_stream)
+                _lib.check(rc, "exposure_apply")
             if gt_ready is not None:
                 torch.cuda.current_stream().wait_event(gt_ready)
             tL, tS = T(False, False, False), T(True, False, False)  # (the L1 gradient is formed in the combine kernel)
@@ -573,12 +660,24 @@ class ViewShardedTrainer:
             g_color = lu._SSIM.backward(tS, self._one)[0]
             # d(lambda_freq * clamp gate * freq_loss) / d image: the scalar rides the regulariser's last backward kernel
             g_freq = _FreqLoss.backward(tF, tT.partials[1])[0] if tF is not None else None
-            with torch.cuda.device(dev):
-                rc = lu._L().hg_training_image_grad(
-                    color.data_ptr(), gt.data_ptr(), g_color.data_ptr(), g_freq.data_ptr() if g_freq is not None else None,
-                    color.numel(), 1.0 - o.lambda_dssim, -o.lambda_dssim, self._one.data_ptr() if g_freq is not None else None,
-                    g_color.data_ptr(), torch.cuda.current_stream().cuda_stream)
-            _lib.check(rc, "training_image_grad")
+            if exp_off is None:
+                with torch.cuda.device(dev):
+                    rc = lu._L().hg_training_image_grad(
+                        color.data_ptr(), gt.data_ptr(), g_color.data_ptr(), g_freq.data_ptr() if g_freq is not None else None,
+                        color.numel(), 1.0 - o.lambda_dssim, -o.lambda_dssim,
+                        self._one.data_ptr() if g_freq is not None else None, g_color.data_ptr(),
+                        torch.cuda.current_stream().cuda_stream)
+                _lib.check(rc, "training_image_grad")
+            else:  # the same gradient through the exposure, + this view's 12 exposure sums into the camera's row
+                H, W = color.size(1), color.size(2)
+                ws = self._exposure_workspace(H, W, dev)
+                with torch.cuda.device(dev):
+                    rc = lu._L().hg_training_image_grad_exposure(
+                        color.data_ptr(), p._exposure.data_ptr() + exp_off, gt.data_ptr(), g_color.data_ptr(),
+                        g_freq.data_ptr() if g_freq is not None else None, H, W, 1.0 - o.lambda_dssim, -o.lambda_dssim,
+                        self._one.data_ptr() if g_freq is not None else None, g_color.data_ptr(),
+                        p.exposure_grad.data_ptr() + exp_off, ws.data_ptr(), torch.cuda.current_stream().cuda_stream)
+                _lib.check(rc, "training_image_grad_exposure")
             g_pd = tN.gd.reshape(plane_depth.shape) if tN is not None else None
             g_am = tN.gam if tN is not None else None
             # the rasterizer's backward leaves the gradient rows of culled Gaussians unwritten: the fused prologue
@@ -590,8 +689,11 @@ class ViewShardedTrainer:
             # kernel over the rendered rows (hg_prologue_backward)
             self._prologue_backward(p, radii, rs, g_xyz, g_sh, g_op, g_sc, g_rot, g_all_map_in,
                                     tSc.grad if tSc is not None else None, tT.partials[2] if tSc is not None else None)
-        return loss, {"visibility_filter": visible, "radii": radii, "means2D_grad": g_means2D,
-                      "num_rendered": int(tR.num_rendered)}
+        out = {"visibility_filter": visible, "radii": radii, "means2D_grad": g_means2D,
+               "num_rendered": int(tR.num_rendered)}
+        if exp_off is not None:
+            out["render"] = image
+        return loss, out
 
     @staticmethod
     def _prologue_backward(p, radii, rs, g_xyz, g_feat, g_op, g_sc, g_rot, g_all_map, g_sc_extra, extra_scale):
@@ -630,12 +732,19 @@ class ViewShardedTrainer:
     def step(self, views, total_views=None):
         """One optimiser step over this rank's `views` = [(camera, gt_image[, gt_ready_event]), ...]; returns the summed
         loss tensor."""
+        if self.train_exposure:
+            for view in views:  # an image without an exposure raises before the step has changed anything
+                self.params.exposure_index(view[0].image_name)
         self.iteration += 1
         timing = getattr(self, "timing", None)  # optional list: (start, views done, step done) CUDA events per step
         if timing is not None:
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             ev[0].record()
         self.params.zero_grad()
+        if self.train_exposure:
+            p = self.params
+            p.exposure_grad.zero_()  # (n x 48 bytes; the views add their sums into it)
+            p._exposure.grad = p.exposure_grad
         total = None
         self.last_view_costs = []
         # optional (`self.time_views = True`): one CUDA event per view boundary, read back by last_view_ms()
@@ -680,6 +789,8 @@ class ViewShardedTrainer:
                 dist.all_reduce(self.params.grad_arena, op=dist.ReduceOp.SUM, group=self.group)
             if self.sparse_adam:  # union of the ranks' visible sets
                 dist.all_reduce(self.visible, op=dist.ReduceOp.MAX, group=self.group)
+            if self.train_exposure:
+                dist.all_reduce(self.params.exposure_grad, op=dist.ReduceOp.SUM, group=self.group)
             if total_views is not None:
                 n_views = total_views
             else:  # ranks may hold uneven shards of views[rank::world]: count what was really rendered
@@ -687,12 +798,39 @@ class ViewShardedTrainer:
                 dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=self.group)
                 n_views = int(round(float(cnt.item())))
         self.adam.step(grad_scale=1.0 / max(n_views, 1), visible_mask=self.visible if self.sparse_adam else None)
+        if self.train_exposure:
+            self._exposure_adam_step(1.0 / max(n_views, 1))
         if getattr(self, "densify", False):
             self._density_schedule()
         if timing is not None:
             ev[2].record()
             timing.append(ev)
         return total
+
+    def _exposure_workspace(self, H, W, dev):
+        """Workspace of hg_training_image_grad_exposure, zero-filled once and grown when a larger image comes (the kernel
+        leaves its counter at zero again after every call)."""
+        need = int(lu._L().hg_exposure_grad_workspace_bytes(H, W))
+        if self._exposure_ws is None or self._exposure_ws.numel() < need:
+            self._exposure_ws = torch.zeros(need, dtype=torch.uint8, device=dev)
+        return self._exposure_ws
+
+    @torch.no_grad()
+    def _exposure_adam_step(self, grad_scale):
+        """hierarchical-3DGS's exposure_optimizer (torch.optim.Adam([_exposure]), eps 1e-8) with its lr set from
+        exposure_scheduler_args(iteration): dense over the whole table (rows of images not in the step keep moving on
+        their moments), its own step count, the gradient scaled by 1 / views as the Gaussians' is."""
+        p = self.params
+        if self.exposure_exp_avg.shape != p._exposure.shape:
+            raise RuntimeError("the exposure table was replaced after the trainer was built (setup_exposures)")
+        self.exposure_step_count += 1
+        n = p._exposure.size(0)
+        with torch.cuda.device(p.param_arena.device):
+            rc = _G().hg_adam_step(p._exposure.data_ptr(), p.exposure_grad.data_ptr(), self.exposure_exp_avg.data_ptr(),
+                                   self.exposure_exp_avg_sq.data_ptr(), n, 12, None, None, 0,
+                                   float(self.exposure_lr(self.iteration)), 0.9, 0.999, 1e-8, self.exposure_step_count,
+                                   float(grad_scale), 0, 0.0, torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "adam_step")
 
     def _zero_densification_stats(self):
         dev, N = self.params.param_arena.device, self.params.N

@@ -60,6 +60,27 @@ HG_API int hg_freq_total(const float *freq_loss, const float *scale_loss, const 
 HG_API int hg_training_image_grad(const float *color, const float *gt, const float *g_ssim, const float *g_freq,
                                   int64_t n, float w_l1, float w_ssim, const float *w_freq, float *out, void *stream);
 
+/* Learned per-image exposure (the reference's render(..., use_trained_exp=True), gaussian_renderer/__init__.py:181-184;
+ * definition in DESIGN.md §3).  exposure12: DEVICE pointer to E [3, 4] row major (12 contiguous floats; the host never
+ * reads it).  Per pixel of color [3, H, W]:
+ *   e[ch] = sum_c color[c] * E[c][ch] + E[ch][3]        (torch.matmul(img.permute(1, 2, 0), E[:3, :3]) + E[:3, 3])
+ * hg_exposure_apply:  out = clamp(e, 0, 1)  (out may alias color).
+ * hg_training_image_grad_exposure:  hg_training_image_grad on the exposed image, taken through the exposure:
+ *   ge  = [0 <= e <= 1] * ( w_l1 * sign(clamp(e, 0, 1) - gt) / (3 H W)  +  w_ssim * g_ssim  +  w_freq[0] * g_freq )
+ *   out[c] = sum_ch E[c][ch] * ge[ch]                   (out may alias g_ssim or g_freq)
+ *   exposure_grad12[c][ch] += sum_pixels color[c] * ge[ch],   exposure_grad12[ch][3] += sum_pixels ge[ch]
+ * The sums are deterministic (grid fixed by H * W, per-CTA partials, fixed-order final sum in double by the last CTA)
+ * and ADDED to exposure_grad12.  workspace: hg_exposure_grad_workspace_bytes(H, W) bytes, zero-filled before its first
+ * use; every call leaves its ticket counter at zero again, so one workspace serves any later call of the same or a
+ * smaller size on the same stream.  With E = eye(3, 4), out equals hg_training_image_grad's bit for bit. */
+HG_API int hg_exposure_apply(const float *color, const float *exposure12, int32_t H, int32_t W, float *out,
+                             void *stream);
+HG_API size_t hg_exposure_grad_workspace_bytes(int32_t H, int32_t W);
+HG_API int hg_training_image_grad_exposure(const float *color, const float *exposure12, const float *gt,
+                                           const float *g_ssim, const float *g_freq, int32_t H, int32_t W, float w_l1,
+                                           float w_ssim, const float *w_freq, float *out, float *exposure_grad12,
+                                           void *workspace, void *stream);
+
 /* Value of the composed training loss of one view (the sum a training loop forms from the reference's pieces:
  * `(1.0 - lambda_dssim) * l1_loss(...) + lambda_dssim * (1.0 - ssim(...))` plus up to two more device scalars, e.g. the
  * total of frequency_regularization_pyramid_scale and the normal term), the Python expression's operations in its
