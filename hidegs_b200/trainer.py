@@ -680,9 +680,11 @@ class ViewShardedTrainer:
                 _lib.check(rc, "training_image_grad_exposure")
             g_pd = tN.gd.reshape(plane_depth.shape) if tN is not None else None
             g_am = tN.gam if tN is not None else None
-            # the rasterizer's backward leaves the gradient rows of culled Gaussians unwritten: the fused prologue
-            # backward below looks at `radii` first (a UAV view culls ~80 % of the slab)
-            tR.skip_culled_rows = True
+            # with the SH sink the rasterizer's backward leaves the gradient rows of culled Gaussians unwritten: the
+            # fused prologue backward below looks at `radii` first (a UAV view culls ~80 % of the slab).  Without the
+            # sink the SH gradient comes back as a dense tensor that the prologue backward adds to the arena row for
+            # row, so every row of it (culled Gaussians, inactive SH bands) must be written
+            tR.skip_culled_rows = tR.sh_sink is not None
             (g_xyz, g_means2D, g_sh, _gc, g_op, g_sc, g_rot, _gcov, g_all_map_in, _n) = _RasterizeGaussians.backward(
                 tR, g_color, None, None, g_am, g_pd, None)
             # all_map backward + scale-regulariser gradient + activation chain rule + accumulation into the arena: one

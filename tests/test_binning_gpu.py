@@ -4,7 +4,9 @@ shared-memory radix sort against the reference's global 64-bit key sort (rasteri
 Bit-exact bar: num_rendered, the sorted 64-bit keys, point_list and the tile ranges — including equal depths
 (the reference's stable sort leaves them in ascending slot order) and lists of every length class the sort
 dispatches on (one warp <= 1024 — packed one-word elements, with the general routine as its fallback —, one CTA <= 2048,
-512-thread CTA <= 12288, HBM scratch beyond)."""
+512-thread CTA <= 12288, HBM scratch beyond).  At every one of them the blend that walks those lists is held to the CPU
+oracle too: colour, contributor counts, final transmittance and observe counts of the forward, and the gradients of the
+backward."""
 import numpy as np
 import pytest
 import torch
@@ -24,7 +26,8 @@ def _forward(case, dev):
 def _check(case, dev, what, min_longest=0, max_longest=None):
     fa, ours = _forward(case, dev)
     so = ru.our_state(ours, case["P"], case["W"], case["H"])
-    oo = ru.oracle_for_case(case).forward()
+    o = ru.oracle_for_case(case)
+    oo = o.forward()
     assert ours[0] == oo["num_rendered"] and ours[0] > 0, what
     rng = oo["ranges"].reshape(-1, 2).astype(np.int64)
     longest = int((rng[:, 1] - rng[:, 0]).max())
@@ -35,6 +38,21 @@ def _check(case, dev, what, min_longest=0, max_longest=None):
     assert np.array_equal(so["point_list"].cpu().numpy().view(np.uint32), oo["point_list"]), what + ": point_list"
     assert np.array_equal(so["ranges"].cpu().numpy().view(np.uint32), oo["ranges"]), what + ": ranges"
     assert np.array_equal(so["keys_unsorted"].cpu().numpy().view(np.uint64), oo["keys_unsorted"]), what + ": emission"
+    # the blend over these lists: the forward's images and per-pixel state (the oracle's expf is the C library's, within
+    # 2 ulp of the GPU's: pixel values agree to ~1e-6, alpha decisions and so contributor counts exactly) ...
+    img = lambda t: torch.as_tensor(t).double().cpu()  # noqa: E731
+    for name, a, b in (("colour", ours[1], oo["color"]), ("all_map", ours[4], oo["all_map"]),
+                       ("final_T", so["final_T"], oo["final_T"])):
+        err = float((img(a) - img(b)).abs().max())
+        assert err <= 1e-4, "%s: %s off by %.3g" % (what, name, err)
+    assert np.array_equal(so["n_contrib"].cpu().numpy().view(np.uint32), oo["n_contrib"]), what + ": n_contrib"
+    assert np.array_equal(ours[3].cpu().numpy(), oo["out_observe"]), what + ": out_observe"
+    # ... and the backward's gradients
+    grads = ru.syn.upstream_grads(case["W"], case["H"])
+    ours_b = ru.OUR_C.rasterize_gaussians_backward(*ru.bwd_args(fa, ours, grads, dev))
+    og = o.backward(grads["color"].numpy(), grads["all_map"].numpy(), grads["plane_depth"].numpy(),
+                    grads["invdepth"].numpy())
+    ru.assert_grads_close([g.cpu() for g in ours_b], [torch.from_numpy(og[n]) for n in ru.GRAD_NAMES], what=what)
     if ru.ref_available():
         ref = ru.ref_module().rasterize_gaussians(*fa)
         torch.cuda.synchronize()
@@ -94,6 +112,16 @@ def test_list_length_classes(cuda_device, what, n, scale, lo, hi):
     import math
     case = ru.build_case(n, 64, 48, seed=41, log_scale_mean=math.log(scale))
     _check(case, cuda_device, what, min_longest=lo, max_longest=hi)
+
+
+def test_lists_beyond_shared_memory_low_opacity(cuda_device):
+    """The longest class at opacity 0.02: the transmittance falls slowly, so each pixel's walk goes on for 1079 .. 1732
+    entries (9 .. 14 of the forward's 128-entry batches, up to ~100 of the backward's 16-entry MMA groups) instead of
+    the 24 .. 46 of the default opacities (measured with the oracle)."""
+    import math
+    case = ru.build_case(30000, 64, 48, seed=41, log_scale_mean=math.log(1.2))
+    case["opacity"] = torch.full_like(case["opacity"], 0.02)
+    _check(case, cuda_device, "lists beyond shared memory, opacity 0.02", min_longest=12289)
 
 
 def test_wide_depth_range_short_lists(cuda_device):

@@ -215,187 +215,6 @@ def test_direct_view_executor_matches_autograd(cuda_device, cache_gt):
         (float((diff > 1e-3).float().mean()), float(diff.median()), float(diff.max()))
 
 
-# ----------------------------------------------------------------------------------------------------------------------
-# The step bench.py times (`train`, `train_config3`), against a composition that shares NO code with it: the
-# UNMODIFIED reference rasterizer (oracle/_ref) between the oracle prologue / epilogue (oracle/geometry_oracle, pinned
-# to the reference's get_normal / normal_from_depth_image), the oracle losses (oracle/loss_oracle, pinned to the
-# reference's utils/loss_utils.py and scripts/frequency_regularization.py) with the weights of
-# /root/reference/arguments/__init__.py:105-135 (lambda_dssim 0.2, single_view_weight 0.015; lambda_freq 1e-3,
-# lambda_scale 5e-3, warm-up 1000: frequency_regularization.py:1589-1594), torch autograd, and torch.optim.Adam on
-# the visible rows (OurAdam.step(relevant)).
-def _oracle_composition(sc_raw, cam, gt, bg, dev, iteration, opt, prologue="oracle"):
-    import bench
-    import oracle.loss_oracle as lo
-    from oracle import geometry_oracle as go
-    import raster_utils as ru
-    H, W = gt.shape[-2:]
-    leaves = {k: v.detach().clone().requires_grad_(True) for k, v in sc_raw.items()}
-    xyz, feat = leaves["xyz"], leaves["features"]
-    opacity = torch.sigmoid(leaves["opacity"])                    # gaussian_model.py:132-133
-    scaling = torch.exp(leaves["scaling"])                        # :118-119
-    rotation = torch.nn.functional.normalize(leaves["rotation"])  # :121-123
-    e_i = torch.empty(0, dtype=torch.int32, device=dev)
-    e_f = torch.empty(0, dtype=torch.float32, device=dev)
-    if prologue == "oracle":
-        am = go.input_all_map(xyz, scaling, rotation, cam.world_view_transform, cam.camera_center)
-    else:  # the library's prologue kernel (pinned on its own by tests/test_geometry_gpu.py): same all_map bits as the step
-        from hidegs_b200 import gaussian_renderer as gr
-        am = gr.geometry_all_map(xyz, scaling, rotation, cam.world_view_transform, cam.camera_center)
-    fa = (bg, e_i, e_i, e_f, e_i, xyz, e_f, am, opacity, scaling, rotation, 1.0, e_f, cam.world_view_transform,
-          cam.full_proj_transform, cam.tanfovx, cam.tanfovy, H, W, feat, 3, cam.camera_center, False, True, False, True)
-    color, radii, _obs, out_am, pdepth, _inv = bench.RefAutograd.apply(ru.ref_module(), fa, xyz, feat, opacity, scaling,
-                                                                       rotation, am)
-    visible = radii > 0
-    # losses on the host, through the oracle (torch CPU autograd); the image gradients travel back to the device
-    c_h = color.detach().cpu().requires_grad_(True)
-    am_h = out_am.detach().cpu().requires_grad_(True)
-    pd_h = pdepth.detach().cpu().requires_grad_(True)
-    sc_h = scaling.detach().cpu().requires_grad_(True)
-    gt_h = gt.cpu()
-    image = c_h.clamp(0, 1)                                       # gaussian_renderer/__init__.py:176
-
-    class Shim:
-        get_scaling = sc_h
-    loss = (1.0 - opt.lambda_dssim) * lo.l1_loss(image, gt_h) + opt.lambda_dssim * (1.0 - lo.ssim(image, gt_h))
-    freq, _mask, info = lo.frequency_regularization_pyramid_scale(
-        image, gt_h, Shim, None, cam, visible.cpu(), iteration, lambda_freq=opt.lambda_freq,
-        lambda_scale=opt.lambda_scale, warmup_iterations=opt.freq_warmup_iterations)
-    loss = loss + freq
-    fx = W / (2 * math.tan(cam.FoVx / 2))
-    fy = H / (2 * math.tan(cam.FoVy / 2))
-    K = go.intrinsic_matrix(fx, fy, 0.5 * W, 0.5 * H)
-    image_weight = (1.0 - lo.get_img_grad_weight(gt_h)).clamp(0, 1) ** 2
-    loss = loss + go.normal_consistency_loss(pd_h, am_h, K, image_weight, opt.single_view_weight)
-    loss.backward()
-    heads, grads = [color, out_am, pdepth], [c_h.grad.to(dev), am_h.grad.to(dev), pd_h.grad.to(dev)]
-    if sc_h.grad is not None:
-        heads.append(scaling)
-        grads.append(sc_h.grad.to(dev))
-    torch.autograd.backward(heads, grads)
-    return float(loss.detach()), leaves, visible, info
-
-
-def _compare_step_with_oracle(dev, sc, cam, gt, full_size):
-    import oracle.loss_oracle as lo
-    from oracle import geometry_oracle as go
-    import raster_utils as ru
-    from hidegs_b200 import gaussian_renderer as gr, trainer as tr
-    bg = torch.zeros(3, device=dev)
-    iteration = 2000
-    names = [n for n, _ in tr.GROUPS]
-    raw = None
-
-    def both(opt):
-        nonlocal raw
-        params = tr.GaussianParams.from_scene(sc, dev)
-        raw = {k: v.detach().clone() for k, v in params.leaves.items()}
-        trainer = tr.ViewShardedTrainer(params, bg, opt=opt)
-        params.zero_grad()
-        loss, pkg = trainer.view_step_direct(cam, gt, iteration)
-        want_loss, leaves, visible, info = _oracle_composition(raw, cam, gt, bg, dev, iteration, opt)
-        assert info.get("freq_loss", 0.0) > 0.0 and "scale_loss" in info  # the regulariser terms took part
-        assert torch.equal(pkg["visibility_filter"], visible)            # visibility set: exact
-        got_loss = float(loss)
-        assert abs(got_loss - want_loss) <= 1e-3 * abs(want_loss), (got_loss, want_loss)  # loss: 1e-3 relative
-        ours = [params.grad_arena[params.slices[n]].view(leaves[n].shape).cpu() for n in names]
-        return ours, [leaves[n].grad.cpu() for n in names], leaves, visible, pkg
-
-    # (1) L1 + SSIM + frequency + scale terms (single_view_weight = 0): the 59-float gradient arena within 1e-3
-    #     relative element-wise and 1e-4 in relative L2, per parameter group — the rasterizer tests' criteria.
-    opt_img = type("ImageTerms", (tr.OptimizationParams,), dict(single_view_weight=0.0))
-    ours, theirs, _lv, _vis, _pkg = both(opt_img)
-    #     (At 2M / 1080p the fp32 SSIM maps of the two sides — separable smem convolution vs torch's conv2d — differ in
-    #     the last bits and the per-Gaussian sums of that gradient cancel: measured 1.26e-4 for xyz, hence 3e-4 there.)
-    ru.assert_grads_close(ours, theirs, names=names, what="composed step, image terms",
-                          l2_tol=3e-4 if full_size else 1e-4, max_bad_frac=1e-5 if full_size else 0.0)
-    # (2) every term (the step bench.py times).  The single-view normal term differentiates normalize(cross(P_r - P_l,
-    #     P_t - P_b)) of neighbouring unprojected depths: dL/d(depth map) is a high-pass field of large, sign-alternating
-    #     values, so (a) it amplifies the last-bit differences between two correct fp32 renders of the depth map
-    #     (ours vs the reference: <= 9.5e-7 absolute) to 4.6e-5 relative, and (b) its per-Gaussian sums cancel, which
-    #     amplifies that by another ~10x (measured, tools/compose_diag2.py: same upstream gradient => rasterizer backward
-    #     1.6e-6 and prologue backward 1e-7 from the reference).  Held here to 3e-3 relative L2; the term's own kernel is
-    #     held tightly in (3) on identical maps.
-    opt = tr.OptimizationParams
-    ours, theirs, leaves, visible, pkg = both(opt)
-    for n, a, b in zip(names, ours, theirs):
-        l2 = float((a.double() - b.double()).norm() / b.double().norm())
-        assert l2 <= 3e-3, ("composed step", n, l2)
-    # (3) the normal term's value and upstream gradients (the kernel view_step_direct runs) against the oracle's autograd
-    #     on the SAME rendered maps: 1e-4 relative L2.
-    H, W = gt.shape[-2:]
-    with torch.no_grad():
-        p3 = tr.GaussianParams.from_scene(sc, dev)
-        maps = gr._render_impl(cam, p3, tr.PipelineParams, bg, _visibility_as_mask=True)
-    pd, am = maps["plane_depth"].detach(), maps["out_all_map"].detach()
-    iw = (1.0 - lo.get_img_grad_weight(gt.cpu())).clamp(0, 1) ** 2
-    K = go.intrinsic_matrix(W / (2 * math.tan(cam.FoVx / 2)), H / (2 * math.tan(cam.FoVy / 2)), 0.5 * W, 0.5 * H)
-    pd_h, am_h = pd.cpu().requires_grad_(True), am.cpu().requires_grad_(True)
-    want_n = go.normal_consistency_loss(pd_h, am_h, K, iw, opt.single_view_weight)
-    want_n.backward()
-    pd_d, am_d = pd.clone().requires_grad_(True), am.clone().requires_grad_(True)
-    got_n = gr.normal_consistency_loss(pd_d, am_d, cam, iw.to(dev), opt.single_view_weight)
-    got_n.backward()
-    assert abs(float(got_n) - float(want_n)) <= 1e-5 * abs(float(want_n))
-    for a, b, n in ((pd_d.grad, pd_h.grad, "plane_depth"), (am_d.grad, am_h.grad, "all_map")):
-        l2 = float((a.double().cpu() - b.double()).norm() / b.double().norm())
-        assert l2 <= 1e-4, ("normal term upstream gradient", n, l2)
-    # one optimiser step: torch.optim.Adam on the visible rows (OurAdam.step(relevant)) vs the arena Adam
-    p2 = tr.GaussianParams.from_scene(sc, dev)
-    t2 = tr.ViewShardedTrainer(p2, bg, start_iteration=iteration - 1)
-    t2.step([(cam, gt)])
-    lrs = dict(xyz=opt.position_lr_init, opacity=opt.opacity_lr, scaling=opt.scaling_lr, rotation=opt.rotation_lr)
-    for n in names:
-        p = torch.nn.Parameter(raw[n].clone())
-        p.grad = leaves[n].grad.clone()
-        if n == "features":  # dc at feature_lr, the rest at feature_lr / 20 (GaussianModel.training_setup)
-            dc, rest = torch.nn.Parameter(p.data[:, :1].clone()), torch.nn.Parameter(p.data[:, 1:].clone())
-            dc.grad, rest.grad = p.grad[:, :1].clone(), p.grad[:, 1:].clone()
-            torch.optim.Adam([{"params": [dc], "lr": opt.feature_lr}, {"params": [rest], "lr": opt.feature_lr / 20.0}],
-                             eps=1e-15).step()
-            stepped = torch.cat([dc.data, rest.data], dim=1)
-        else:
-            torch.optim.Adam([p], lr=lrs[n], eps=1e-15).step()
-            stepped = p.data
-        want = torch.where(visible.view(-1, *([1] * (stepped.dim() - 1))), stepped, raw[n])
-        got = p2.leaves[n].detach()
-        assert torch.equal(got[~visible], raw[n][~visible]), n      # rows outside the visible set are untouched
-        # (the first Adam step moves every element by lr * g / (|g| + eps) ~ lr * sign(g): where a gradient sits at the
-        # blend's atomic-order noise level the sign may differ, so the bulk is held tightly and the tail loosely)
-        diff = (got - want).abs()
-        lr = opt.feature_lr if n == "features" else lrs[n]
-        frac_off = float((diff > 0.05 * lr).float().mean())
-        assert frac_off <= 2e-3, (n, frac_off, float(diff.max()))
-        assert float(diff.max()) <= 2.0 * lr * 1.0001 + 1e-12, (n, float(diff.max()))
-
-
-def test_step_vs_oracle_composition(cuda_device):
-    """view_step_direct (the step `bench.py` times) against the reference rasterizer + oracle losses + torch Adam on
-    the 30k / 320x208 scene: loss 1e-3, visibility set exact, gradient arena 1e-3 element-wise / 1e-4 relative L2 for
-    the image terms and 3e-3 with the (ill-conditioned) normal term, whose kernel is held to 1e-4 on identical maps;
-    parameters after one optimiser step."""
-    import raster_utils as ru
-    if not ru.ref_available():
-        pytest.skip("reference rasterizer not built")
-    dev = cuda_device
-    sc, cams, gts, _tr = _setup(dev)
-    _compare_step_with_oracle(dev, sc, cams[0], gts[0], full_size=False)
-
-
-def test_step_vs_oracle_composition_2m_1080p(cuda_device):
-    """Same comparison at BASELINE configs[3]: 2M Gaussians (config-2 recipe), one 1920x1080 view."""
-    import raster_utils as ru
-    from hidegs_b200 import synthetic as syn
-    if not ru.ref_available():
-        pytest.skip("reference rasterizer not built")
-    dev = cuda_device
-    sc = syn.make_scene(2_000_000, seed=0)
-    cam = syn.default_camera(1920, 1080).to(dev)
-    g = torch.Generator().manual_seed(11)
-    gt = torch.nn.functional.avg_pool2d(torch.rand(1, 3, 1080, 1920, generator=g), 5, stride=1, padding=2)[0].clamp(0, 1).to(dev)
-    _compare_step_with_oracle(dev, sc, cam, gt, full_size=True)
-    torch.cuda.empty_cache()
-
-
 def test_gaussian_count_not_multiple_of_four(cuda_device):
     """The arenas pad every parameter group to 16 bytes: a step with N = 4k + 1 Gaussians runs on the fused path and
     matches the autograd path."""
