@@ -5,7 +5,7 @@ from . import _lib
 
 EXPORTED_SYMBOLS = (
     "hg_reduce_workspace_bytes", "hg_l1_loss", "hg_l2_loss", "hg_pixel_loss_backward", "hg_freq_total", "hg_training_image_grad", "hg_exposure_apply", "hg_exposure_grad_workspace_bytes",
-    "hg_training_image_grad_exposure", "hg_training_loss_value", "hg_ssim_workspace_bytes", "hg_ssim", "hg_ssim_backward",
+    "hg_training_image_grad_exposure", "hg_invdepth_l1_workspace_bytes", "hg_invdepth_l1", "hg_training_loss_value", "hg_ssim_workspace_bytes", "hg_ssim", "hg_ssim_backward",
     "hg_ssim_window_workspace_bytes", "hg_ssim_window", "hg_ssim_window_backward",
     "hg_img_grad_weight_workspace_bytes", "hg_img_grad_weight", "hg_lncc", "hg_lncc_backward",
     "hg_scale_reg_workspace_bytes", "hg_scale_reg", "hg_fft2_workspace_bytes", "hg_fft2_r2c", "hg_fft2_c2r",
@@ -31,6 +31,8 @@ def lib():
         "hg_exposure_apply": (ctypes.c_int, [vp, vp, i32, i32, vp, vp]),
         "hg_exposure_grad_workspace_bytes": (sz, [i32, i32]),
         "hg_training_image_grad_exposure": (ctypes.c_int, [vp, vp, vp, vp, vp, i32, i32, f32, f32, vp, vp, vp, vp, vp]),
+        "hg_invdepth_l1_workspace_bytes": (sz, [i32, i32]),
+        "hg_invdepth_l1": (ctypes.c_int, [vp, vp, vp, i32, i32, f32, vp, vp, vp, vp, vp]),
         "hg_training_loss_value": (ctypes.c_int, [vp, vp, vp, vp, f32, vp, vp]),
         "hg_ssim_workspace_bytes": (sz, [i32, i32, i32, i32]),
         "hg_ssim": (ctypes.c_int, [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp]),

@@ -155,6 +155,51 @@ def ssim(img1, img2, window_size=11, size_average=True):
     return _SSIM.apply(img1, img2, size_average, window_size)
 
 
+def _invdepth_l1_launch(invdepth, mono, mask, weight, grad, value, loss_inout, ws):
+    """hg_invdepth_l1 on contiguous [.., H, W] fp32 CUDA tensors (mask may be None, loss_inout may be None)."""
+    H, W = invdepth.shape[-2:]
+    with torch.cuda.device(invdepth.device):
+        rc = _L().hg_invdepth_l1(invdepth.data_ptr(), mono.data_ptr(), mask.data_ptr() if mask is not None else None,
+                                 H, W, float(weight), grad.data_ptr(), value.data_ptr(),
+                                 loss_inout.data_ptr() if loss_inout is not None else None, ws.data_ptr(), _stream())
+    _lib.check(rc, "invdepth_l1")
+
+
+class _InvDepthL1(torch.autograd.Function):
+    """mean |(invdepth - mono) * mask|: value and unit-weight gradient in one pass (hg_invdepth_l1); the backward scales
+    that gradient by the upstream scalar.  The prior and the mask receive no gradient."""
+
+    @staticmethod
+    def forward(ctx, invdepth, mono, mask):
+        ts = (invdepth, mono) + ((mask,) if mask is not None else ())
+        _check_cuda(*ts)
+        if any(t.shape != invdepth.shape for t in ts) or invdepth.dim() < 2 or invdepth.numel() != \
+                invdepth.size(-1) * invdepth.size(-2):
+            raise RuntimeError("inverse_depth_l1: expected [1, H, W] / [H, W] tensors of one shape, got %s"
+                               % [tuple(t.shape) for t in ts])
+        x, m = invdepth.contiguous(), mono.contiguous()
+        k = mask.contiguous() if mask is not None else None
+        H, W = x.shape[-2:]
+        grad = torch.empty_like(x)
+        value = torch.empty((), dtype=torch.float32, device=x.device)
+        ws = torch.zeros(int(_L().hg_invdepth_l1_workspace_bytes(H, W)), dtype=torch.uint8, device=x.device)
+        _invdepth_l1_launch(x, m, k, 1.0, grad, value, None, ws)
+        ctx.save_for_backward(grad)
+        return value
+
+    @staticmethod
+    def backward(ctx, g):
+        (grad,) = ctx.saved_tensors
+        return grad * g.detach().reshape(()), None, None
+
+
+def inverse_depth_l1(invdepth, mono, mask=None):
+    """mean_{H,W} |(invdepth - mono) * mask| (graphdeco's Ll1depth without its weight; DESIGN.md §3 "Depth
+    regularisation"): `invdepth` the rendered inverse depth [1, H, W], `mono` the camera's prior, `mask` a float map or
+    None for all ones.  Differentiable w.r.t. `invdepth` only."""
+    return _InvDepthL1.apply(invdepth, mono, mask)
+
+
 def get_img_grad_weight(img, beta=2.0):
     """Edge-aware weight map of an image (used on ground-truth images; returned without autograd history)."""
     _check_cuda(img)

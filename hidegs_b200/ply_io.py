@@ -209,3 +209,50 @@ def load_exposures(path, device="cuda"):
     with open(path, "r") as f:
         exposures = json.load(f)
     return {name: torch.tensor(exposures[name], dtype=torch.float32, device=device) for name in exposures}
+
+
+def load_depth_params(path):
+    """depth_params.json of graphdeco 3DGS's dataset readers: {image_name: {"scale", "offset"}} as a dict whose entries
+    also carry "med_scale", the median of the POSITIVE scales of the file (0 when there are none).  DESIGN.md §3 "Depth
+    regularisation"."""
+    with open(path, "r") as f:
+        params = json.load(f)
+    scales = np.array([float(params[k]["scale"]) for k in params], dtype=np.float64)
+    med_scale = float(np.median(scales[scales > 0])) if (scales > 0).any() else 0.0
+    for k in params:
+        params[k]["med_scale"] = med_scale
+    return params
+
+
+def attach_depth_prior(cam, invdepth, depth_params=None, mask=None, device=None):
+    """Set `cam.invdepthmap`, `cam.depth_mask` and `cam.depth_reliable` as graphdeco 3DGS's Camera.__init__ does from a
+    monocular inverse-depth map ALREADY at render resolution ([H, W] or [1, H, W], H x W = cam.image_height x
+    cam.image_width; a tensor or an array; decoding and resizing are the dataset tooling's): negative values are clamped
+    to 0 first; with `depth_params` (an entry of load_depth_params) the prior is unreliable when scale < 0.2 med_scale or
+    scale > 5 med_scale, which also zeroes the mask, and the map becomes invdepth * scale + offset when scale > 0.
+    `mask`: a float map of the same shape, or None for all ones.  The maps are stored as float32 [1, H, W] on `device`
+    (default: where `invdepth` is; the trainer wants the parameters' device).  Returns `cam`."""
+    H, W = int(cam.image_height), int(cam.image_width)
+
+    def as_map(x, what):
+        t = torch.as_tensor(x)
+        if t.dim() == 2:
+            t = t[None]
+        if tuple(t.shape) != (1, H, W):
+            raise ValueError("attach_depth_prior: %s has shape %s, the camera renders (1, %d, %d)"
+                             % (what, tuple(torch.as_tensor(x).shape), H, W))
+        return t.to(device=device if device is not None else t.device, dtype=torch.float32).contiguous()
+
+    inv = as_map(invdepth, "invdepth").clone()
+    m = as_map(mask, "mask").clone() if mask is not None else None
+    inv[inv < 0] = 0
+    reliable = True
+    if depth_params is not None:
+        scale, offset, med = float(depth_params["scale"]), float(depth_params["offset"]), float(depth_params["med_scale"])
+        if scale < 0.2 * med or scale > 5 * med:
+            reliable = False
+            m = torch.zeros_like(inv) if m is None else m * 0
+        if scale > 0:
+            inv = inv * scale + offset
+    cam.invdepthmap, cam.depth_mask, cam.depth_reliable = inv, m, reliable
+    return cam

@@ -76,6 +76,11 @@ class OptimizationParams:
     exposure_lr_delay_steps = 5000
     exposure_lr_delay_mult = 0.001
     iterations = 30_000
+    # monocular inverse-depth supervision (ViewShardedTrainer(depth_regularization=True)): weight
+    # get_expon_lr_func(depth_l1_weight_init, depth_l1_weight_final, max_steps=iterations) at the trainer's iteration;
+    # graphdeco 3DGS's arguments/__init__.py values as recalled, not checked against a reference tree
+    depth_l1_weight_init = 1.0
+    depth_l1_weight_final = 0.01
 
 
 class _ActivateParams(torch.autograd.Function):
@@ -464,18 +469,24 @@ def balance_views(costs, world, speeds=None):
 
 
 class ViewShardedTrainer:
-    train_exposure = False  # (class default: also read by trainers assembled without __init__)
+    train_exposure = False  # (class defaults: also read by trainers assembled without __init__)
+    depth_regularization = False
 
     def __init__(self, params: GaussianParams, background, opt=OptimizationParams, pipe=PipelineParams, group=None,
                  sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0, densify=False,
-                 scene_extent=None, train_exposure=False):
+                 scene_extent=None, train_exposure=False, depth_regularization=False):
         """`densify`: run the adaptive density control schedule of the OptimizationParams densify_* fields inside
         `step()` (off by default); it needs `scene_extent` (`cameras_extent(cameras)`) and turns the densification
         statistics on.
         `train_exposure`: render every view through the exposure of its `cam.image_name` and learn the table (off by
         default); it needs `params.setup_exposures(image_names)` first.  Every step zeroes the exposure gradient table,
         sums it over the ranks and steps it with its own Adam (eps 1e-8, dense over the whole table, the lr schedule of
-        the OptimizationParams exposure_* fields)."""
+        the OptimizationParams exposure_* fields).
+        `depth_regularization`: add graphdeco's masked inverse-depth L1, w(it) mean |(invdepth - cam.invdepthmap) *
+        cam.depth_mask|, to the loss of every view whose camera carries a reliable prior (ply_io.attach_depth_prior;
+        DESIGN.md §3 "Depth regularisation"), with w(it) the schedule of the OptimizationParams depth_l1_weight_*
+        fields (off by default).  A view without a reliable prior, or a step with w(it) = 0, runs as it does with the
+        flag off."""
         self.params, self.bg, self.opt, self.pipe, self.group = params, background, opt, pipe, group
         if densify and scene_extent is None:
             raise ValueError("densify=True needs scene_extent (cameras_extent(cameras))")
@@ -492,6 +503,12 @@ class ViewShardedTrainer:
             self.exposure_exp_avg_sq = torch.zeros_like(params._exposure, requires_grad=False)
             self.exposure_step_count = 0
             self._exposure_ws = None
+        self.depth_regularization = bool(depth_regularization)
+        if self.depth_regularization:
+            from .optim import get_expon_lr_func
+            self.depth_l1_weight = get_expon_lr_func(opt.depth_l1_weight_init, opt.depth_l1_weight_final,
+                                                     max_steps=opt.iterations)
+            self._depth_ws = None
         self.densify, self.scene_extent = densify, scene_extent
         densification_stats = densification_stats or densify
         self.adam = ArenaAdam(params, opt)
@@ -544,6 +561,12 @@ class ViewShardedTrainer:
             image_weight = cache[2] if cache is not None else (1.0 - lu.get_img_grad_weight(gt)).clamp(0, 1) ** 2
             loss = loss + gr.normal_consistency_loss(pkg["plane_depth"], pkg["out_all_map"], cam, image_weight,
                                                      o.single_view_weight)
+        depth = self._depth_term(cam, iteration)
+        if depth is not None:  # + w(it) * Ll1depth, added last
+            mono, mask, w = depth
+            depth_l1 = lu.inverse_depth_l1(pkg["depth"], mono, mask)
+            loss = loss + w * depth_l1
+            pkg["depth_l1"] = depth_l1.detach()
         return loss, pkg
 
     # ------------------------------------------------------------------------------------------------------------------
@@ -573,9 +596,11 @@ class ViewShardedTrainer:
         """Forward AND backward of one view (gradients accumulated into the arena), without autograd.  Returns
         (loss value tensor, dict with "visibility_filter" (mask), "radii", "means2D_grad" — defined on the rendered rows
         only: the rasterizer's backward does not write the rows of culled Gaussians here); with train_exposure also
-        "render", the exposed, clamped image the losses saw."""
+        "render", the exposed, clamped image the losses saw; with the depth term on this view also "depth_l1", the
+        unweighted masked inverse-depth L1 (device scalar)."""
         o, p, T = self.opt, self.params, self._Tape
         dev = p.param_arena.device
+        depth = self._depth_term(cam, iteration)  # (mono, mask, w) or None: the view runs as with the flag off
         exp_off = None  # byte offset of this camera's exposure row in the table / its gradient table
         if self.train_exposure:
             exp_off = 48 * p.exposure_index(cam.image_name)
@@ -653,6 +678,13 @@ class ViewShardedTrainer:
                     normal_term.data_ptr() if normal_term is not None else None, float(o.lambda_dssim), loss.data_ptr(),
                     torch.cuda.current_stream().cuda_stream)
             _lib.check(rc, "training_loss_value")
+            g_inv = depth_l1 = None
+            if depth is not None:  # + w(it) mean |(invdepth - mono) * mask| onto `loss`, and its gradient, in one pass
+                mono, mask, w = depth
+                g_inv = torch.empty_like(_inv)
+                depth_l1 = torch.empty((), dtype=torch.float32, device=dev)
+                lu._invdepth_l1_launch(_inv, mono, mask, w, g_inv, depth_l1, loss,
+                                       self._depth_workspace(_inv.size(-2), _inv.size(-1), dev))
             # ---- backward (upstream gradient of the loss = 1)
             # dL/dcolor = [0 <= color <= 1] ((1 - l) dL1 - l dSSIM + gate lf dfreq) in ONE pass over the image
             if self._one is None:
@@ -686,7 +718,7 @@ class ViewShardedTrainer:
             # row, so every row of it (culled Gaussians, inactive SH bands) must be written
             tR.skip_culled_rows = tR.sh_sink is not None
             (g_xyz, g_means2D, g_sh, _gc, g_op, g_sc, g_rot, _gcov, g_all_map_in, _n) = _RasterizeGaussians.backward(
-                tR, g_color, None, None, g_am, g_pd, None)
+                tR, g_color, None, None, g_am, g_pd, g_inv)
             # all_map backward + scale-regulariser gradient + activation chain rule + accumulation into the arena: one
             # kernel over the rendered rows (hg_prologue_backward)
             self._prologue_backward(p, radii, rs, g_xyz, g_sh, g_op, g_sc, g_rot, g_all_map_in,
@@ -695,6 +727,8 @@ class ViewShardedTrainer:
                "num_rendered": int(tR.num_rendered)}
         if exp_off is not None:
             out["render"] = image
+        if depth_l1 is not None:
+            out["depth_l1"] = depth_l1
         return loss, out
 
     @staticmethod
@@ -737,6 +771,9 @@ class ViewShardedTrainer:
         if self.train_exposure:
             for view in views:  # an image without an exposure raises before the step has changed anything
                 self.params.exposure_index(view[0].image_name)
+        if self.depth_regularization:
+            for view in views:  # a prior the step cannot use raises before the step has changed anything
+                self._depth_prior(view[0])
         self.iteration += 1
         timing = getattr(self, "timing", None)  # optional list: (start, views done, step done) CUDA events per step
         if timing is not None:
@@ -808,6 +845,46 @@ class ViewShardedTrainer:
             ev[2].record()
             timing.append(ev)
         return total
+
+    def _depth_prior(self, cam):
+        """(invdepthmap, depth_mask or None) of the camera when it carries a reliable prior, else None.  ValueError
+        for a prior this trainer cannot use: not a float32 [1, H, W] tensor at the camera's resolution on the
+        parameters' device."""
+        mono = getattr(cam, "invdepthmap", None)
+        if mono is None or not getattr(cam, "depth_reliable", True):
+            return None
+        mask = getattr(cam, "depth_mask", None)
+        shape = (1, int(cam.image_height), int(cam.image_width))
+        dev = self.params.param_arena.device
+        for what, t in (("invdepthmap", mono), ("depth_mask", mask)):
+            if t is None:
+                continue
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or tuple(t.shape) != shape:
+                raise ValueError("camera %r: %s must be a float32 tensor of shape %s, got %s"
+                                 % (getattr(cam, "image_name", None), what, shape,
+                                    (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t)))
+            if t.device != dev:
+                raise ValueError("camera %r: %s is on %s, the parameters on %s"
+                                 % (getattr(cam, "image_name", None), what, t.device, dev))
+        return mono.contiguous(), mask.contiguous() if mask is not None else None
+
+    def _depth_term(self, cam, iteration):
+        """(mono, mask, w(iteration)) when the depth term applies to this view, else None."""
+        if not self.depth_regularization:
+            return None
+        prior = self._depth_prior(cam)
+        if prior is None:
+            return None
+        w = float(self.depth_l1_weight(iteration))
+        return prior + (w,) if w != 0.0 else None
+
+    def _depth_workspace(self, H, W, dev):
+        """Workspace of hg_invdepth_l1, zero-filled once and grown when a larger image comes (the kernel leaves its
+        counter at zero again after every call)."""
+        need = int(lu._L().hg_invdepth_l1_workspace_bytes(H, W))
+        if self._depth_ws is None or self._depth_ws.numel() < need:
+            self._depth_ws = torch.zeros(need, dtype=torch.uint8, device=dev)
+        return self._depth_ws
 
     def _exposure_workspace(self, H, W, dev):
         """Workspace of hg_training_image_grad_exposure, zero-filled once and grown when a larger image comes (the kernel

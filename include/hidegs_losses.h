@@ -81,6 +81,21 @@ HG_API int hg_training_image_grad_exposure(const float *color, const float *expo
                                            float w_ssim, const float *w_freq, float *out, float *exposure_grad12,
                                            void *workspace, void *stream);
 
+/* Monocular inverse-depth supervision (graphdeco 3DGS / hierarchical-3DGS's `Ll1depth`; definition in DESIGN.md §3
+ * "Depth regularisation").  invdepth: the rasterizer's inverse depth [H, W]; mono: the camera's prior [H, W]; mask:
+ * [H, W] fp32 or NULL (all ones).  One streaming pass:
+ *   d = (invdepth - mono) * mask
+ *   grad[p] = (weight / (H W)) * sgn(d[p]) * mask[p]          (sgn(0) = 0; weight * (1 / (H W)) rounded in fp32)
+ *   value[0] = mean |d|  (unweighted)                         loss_inout[0] += weight * value[0]  (when not NULL)
+ * The sum is deterministic (grid fixed by H * W, per-CTA partials, fixed-order final sum in double by the last CTA) and
+ * does not depend on the alignment of the pointers.  weight is a host float: no host read, no synchronisation.
+ * workspace: hg_invdepth_l1_workspace_bytes(H, W) bytes, zero-filled before its first use; every call leaves its
+ * ticket counter at zero again, so one workspace serves any later call of the same or a smaller size on the same
+ * stream. */
+HG_API size_t hg_invdepth_l1_workspace_bytes(int32_t H, int32_t W);
+HG_API int hg_invdepth_l1(const float *invdepth, const float *mono, const float *mask, int32_t H, int32_t W,
+                          float weight, float *grad, float *value, float *loss_inout, void *workspace, void *stream);
+
 /* Value of the composed training loss of one view (the sum a training loop forms from the reference's pieces:
  * `(1.0 - lambda_dssim) * l1_loss(...) + lambda_dssim * (1.0 - ssim(...))` plus up to two more device scalars, e.g. the
  * total of frequency_regularization_pyramid_scale and the normal term), the Python expression's operations in its
