@@ -310,18 +310,26 @@ preprocess_fwd_kernel(const int P, const int N, const int D, const int M,
   const bool need_sh = (colors_precomp == nullptr);
   if (need_sh) {
     const int row = M * 3;
-    // Fast path: rows of this warp are contiguous -> coalesced staging.
+    // Fast path: rows of this warp are contiguous -> coalesced staging.  The float4 staging skips the float4s of
+    // culled rows, which is only exact when no float4 straddles two rows (row % 4 == 0), and needs 16-byte aligned
+    // shs; other widths and misaligned views are staged float by float.  Either way the colour comes from the one
+    // eval_sh below, so a view of the same rows at another alignment gives the same bits.
     const bool staged = (indices == nullptr) && (parent_indices == nullptr);
     if (staged) {
       const unsigned any = __ballot_sync(0xffffffffu, alive);
       if (any) {
         const int stride = row | 1;
         const int warp_first = blockIdx.x * kThreads + warp * 32;
-        const size_t base = (size_t)warp_first * row;         // float index, multiple of 4
+        const size_t base = (size_t)warp_first * row;         // float index of the warp's first row
         const size_t total = (size_t)N * row;
         float* dst = s_sh[warp];
-        if (row == 48) stage_sh_rows<48>(shs, base, total, row, lane, dst, any);  // rows of culled slots are skipped
-        else stage_sh_rows<0>(shs, base, total, row, lane, dst, any);
+        // rows of culled slots are skipped
+        if ((row & 3) == 0 && (reinterpret_cast<uintptr_t>(shs) & 15) == 0) {
+          if (row == 48) stage_sh_rows<48>(shs, base, total, row, lane, dst, any);
+          else stage_sh_rows<0>(shs, base, total, row, lane, dst, any);
+        } else {
+          stage_sh_rows_scalar(shs, base, total, row, lane, dst, any);
+        }
         __syncwarp();
         if (alive) {
           const float cx = __ldg(campos), cy = __ldg(campos + 1), cz = __ldg(campos + 2);

@@ -139,6 +139,10 @@ static int validate(const hg_raster_inputs* in) {
     set_error("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!");
     return HG_ERR_INVALID_ARG;
   }
+  if (reinterpret_cast<uintptr_t>(in->rotations) & 15) {  // read as one float4 per Gaussian
+    set_error("rotations must be 16-byte aligned (got %p)", (const void*)in->rotations);
+    return HG_ERR_INVALID_ARG;
+  }
   if (in->shs && (in->M <= 0 || in->M > 16 || in->D < 0 || (in->D + 1) * (in->D + 1) > in->M)) {
     set_error("SH degree %d does not fit %d coefficients (max 16)", in->D, in->M);
     return HG_ERR_INVALID_ARG;

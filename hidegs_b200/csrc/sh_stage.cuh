@@ -6,7 +6,9 @@
 namespace hg {
 
 // Warp-cooperative, coalesced load of 32 consecutive SH rows into shared memory
-// (row-major, odd stride).  ROW > 0 fixes the row length at compile time.
+// (row-major, odd stride).  ROW > 0 fixes the row length at compile time.  The row length must be a multiple of 4
+// and `shs + base` 16-byte aligned (checked by the caller): the loads are float4s, and the float4s of rows whose bit
+// in `row_mask` is clear are skipped, which leaves no live float unloaded only when no float4 straddles two rows.
 template <int ROW>
 __device__ __forceinline__ void stage_sh_rows(const float* __restrict__ shs, size_t base,
                                               size_t total, int row_rt, int lane, float* dst,
@@ -50,6 +52,28 @@ __device__ __forceinline__ void stage_sh_rows(const float* __restrict__ shs, siz
   }
 }
 
+// The same for any row length and alignment: one float per lane and step (still coalesced), each loaded only when
+// its own row's bit in `row_mask` is set; kGroup independent loads are in flight before any is stored.
+__device__ __forceinline__ void stage_sh_rows_scalar(const float* __restrict__ shs, size_t base, size_t total, int row,
+                                                     int lane, float* dst, uint32_t row_mask) {
+  const int stride = row | 1;
+  const int nfloat = 32 * row;
+  constexpr int kGroup = 4;
+#pragma unroll 1
+  for (int i0 = lane; i0 < nfloat; i0 += 32 * kGroup) {
+    float val[kGroup];
+#pragma unroll
+    for (int u = 0; u < kGroup; ++u) {
+      const int i = i0 + 32 * u;
+      val[u] = (i < nfloat && ((row_mask >> (i / row)) & 1u) && base + i < total) ? __ldg(shs + base + i) : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < kGroup; ++u) {
+      const int i = i0 + 32 * u;
+      if (i < nfloat) dst[(i / row) * stride + i % row] = val[u];
+    }
+  }
+}
 
 // The inverse: rows of the tile -> global, coalesced float4 stores.  Rows whose bit in `row_mask` is clear are
 // written as zeros if `zero_others`, else left untouched.  `row` must be a multiple of 4 and `dst + base` 16-byte

@@ -53,6 +53,13 @@ torch::Tensor f32(const torch::Tensor& t, const char* name) {
                 t.scalar_type(), " on ", t.device());
   return t.contiguous();
 }
+// The library reads rotations as one float4 per row; a contiguous view that starts off a 16-byte boundary (e.g.
+// params[1:]) is copied into fresh storage so that the drop-in API keeps accepting it.
+torch::Tensor f32_aligned16(const torch::Tensor& t, const char* name) {
+  torch::Tensor c = f32(t, name);
+  if (c.defined() && c.numel() != 0 && reinterpret_cast<uintptr_t>(c.data_ptr()) % 16 != 0) return c.clone();
+  return c;
+}
 torch::Tensor i32(const torch::Tensor& t, const char* name) {
   if (!t.defined()) return t;
   if (t.numel() != 0)
@@ -165,7 +172,7 @@ rasterize_gaussians(torch::Tensor background, torch::Tensor indices, torch::Tens
   background = f32(background, "bg"); viewmatrix = f32(viewmatrix, "viewmatrix"); projmatrix = f32(projmatrix, "projmatrix");
   campos = f32(campos, "campos"); means3D = f32(means3D, "means3D"); colors = f32(colors, "colors_precomp");
   all_map = f32(all_map, "all_map"); opacity = f32(opacity, "opacities"); scales = f32(scales, "scales");
-  rotations = f32(rotations, "rotations"); cov3D_precomp = f32(cov3D_precomp, "cov3D_precomp"); sh = f32(sh, "shs");
+  rotations = f32_aligned16(rotations, "rotations"); cov3D_precomp = f32(cov3D_precomp, "cov3D_precomp"); sh = f32(sh, "shs");
   ts = f32(ts, "interpolation_weights");
   indices = i32(indices, "render_indices"); parent_indices = i32(parent_indices, "parent_indices");
   kids = i32(kids, "num_node_kids");
@@ -255,7 +262,7 @@ py::tuple rasterize_gaussians_backward(torch::Tensor background, torch::Tensor a
   background = f32(background, "bg"); viewmatrix = f32(viewmatrix, "viewmatrix"); projmatrix = f32(projmatrix, "projmatrix");
   campos = f32(campos, "campos"); means3D = f32(means3D, "means3D"); colors = f32(colors, "colors_precomp");
   all_maps = f32(all_maps, "all_map"); opacities = f32(opacities, "opacities"); scales = f32(scales, "scales");
-  rotations = f32(rotations, "rotations"); cov3D_precomp = f32(cov3D_precomp, "cov3D_precomp"); sh = f32(sh, "shs");
+  rotations = f32_aligned16(rotations, "rotations"); cov3D_precomp = f32(cov3D_precomp, "cov3D_precomp"); sh = f32(sh, "shs");
   ts = f32(ts, "interpolation_weights"); all_map_pixels = f32(all_map_pixels, "all_map_pixels");
   indices = i32(indices, "render_indices"); parent_indices = i32(parent_indices, "parent_indices");
   kids = i32(kids, "num_node_kids"); radii = i32(radii, "radii");

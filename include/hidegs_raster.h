@@ -95,7 +95,8 @@ typedef struct hg_raster_inputs {
   const float *all_map;        /* [P,5] or NULL                           */
   const float *opacities;      /* [N,1]                                   */
   const float *scales;         /* [N,3] or NULL                           */
-  const float *rotations;      /* [N,4] or NULL                           */
+  const float *rotations;      /* [N,4] or NULL; 16-byte aligned (read as one float4 per row;
+                                  forward and backward return HG_ERR_INVALID_ARG otherwise) */
   const float *cov3D_precomp;  /* [N,6] or NULL                           */
 } hg_raster_inputs;
 

@@ -14,14 +14,14 @@ from hidegs_b200.diff_gaussian_rasterization import _C as OUR_C  # noqa: E402
 
 # --------------------------------------------------------------------- scenes
 def build_case(n, W, H, seed=0, log_scale_mean=None, device="cpu", sh_degree=3, with_hier=False,
-               with_indices=False, eye=(0.0, 0.0, -5.0)):
+               with_indices=False, eye=(0.0, 0.0, -5.0), sh_coeffs=16):
     """Synthetic scene + camera + all_map (+ optional hierarchy inputs), CPU tensors."""
     import math
     cam = syn.default_camera(W, H, eye=eye)
     if log_scale_mean is None:
         # keep the splat footprint in pixels similar to config 2 (sigma ~ 3 px at 1080p)
         log_scale_mean = math.log(0.01 * 1920.0 / W)
-    sc = syn.make_scene(n, seed=seed, log_scale_mean=log_scale_mean)
+    sc = syn.make_scene(n, seed=seed, log_scale_mean=log_scale_mean, sh_coeffs=sh_coeffs)
     g = torch.Generator().manual_seed(seed + 1000)
     case = dict(cam=cam, W=W, H=H, sh_degree=sh_degree, **sc)
     P = n
@@ -250,8 +250,10 @@ def assert_grads_close(ours, theirs, names=GRAD_NAMES, rtol=1e-3, floor=None, l2
             what, name, 100 * frac, float((a - b).abs().max()), scale)
 
 
-def oracle_for_case(case, render_geo=True, do_depth=True, bg=(0.1, 0.2, 0.3), colors_precomp=None, nthreads=1):
-    """CPU oracle (oracle/raster_oracle.py) configured like op_args()."""
+def oracle_for_case(case, render_geo=True, do_depth=True, bg=(0.1, 0.2, 0.3), colors_precomp=None, nthreads=1,
+                    scale_modifier=1.0, cov3D_precomp=None):
+    """CPU oracle (oracle/raster_oracle.py) configured like op_args().  With `cov3D_precomp` the scales and rotations
+    are left out, as render() does when it precomputes the covariance."""
     from oracle.raster_oracle import OracleRasterizer
     cam = case["cam"]
     n = lambda k: case[k].numpy() if k in case else None  # noqa: E731
@@ -261,7 +263,10 @@ def oracle_for_case(case, render_geo=True, do_depth=True, bg=(0.1, 0.2, 0.3), co
         opacities=case["opacity"].numpy(), image_height=case["H"], image_width=case["W"], tanfovx=cam.tanfovx,
         tanfovy=cam.tanfovy, shs=case["shs"].numpy() if colors_precomp is None else None,
         colors_precomp=None if colors_precomp is None else colors_precomp.numpy(), all_map=case["all_map"].numpy(),
-        scales=case["scales"].numpy(), rotations=case["rotations"].numpy(), sh_degree=case["sh_degree"],
+        scales=None if cov3D_precomp is not None else case["scales"].numpy(),
+        rotations=None if cov3D_precomp is not None else case["rotations"].numpy(),
+        cov3D_precomp=None if cov3D_precomp is None else cov3D_precomp.numpy(), scale_modifier=scale_modifier,
+        sh_degree=case["sh_degree"],
         render_indices=n("render_indices"), parent_indices=n("parent_indices"),
         interpolation_weights=n("interpolation_weights"), num_node_kids=n("num_node_kids"), render_geo=render_geo,
         do_depth=do_depth, nthreads=nthreads)

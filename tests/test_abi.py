@@ -81,6 +81,35 @@ def test_forward_validates_before_touching_the_gpu():
     s.D = 4  # degree 4 does not fit 16 coefficients
     rc = lib.hg_raster_forward(ctypes.byref(s), cb, None, cb, None, cb, None, 1, None, 1, 1, 1, 1, ctypes.byref(r), None)
     assert rc == 1 and b"SH degree" in lib.hg_last_error()
+    # rotations are read as float4: a pointer off a 16-byte boundary is refused (one float into a row, or 8 bytes)
+    s.D = 3
+    for bad in (260, 264):
+        s.rotations = bad
+        rc = lib.hg_raster_forward(ctypes.byref(s), cb, None, cb, None, cb, None, 1, None, 1, 1, 1, 1, ctypes.byref(r),
+                                   None)
+        assert rc == 1 and b"rotations must be 16-byte aligned" in lib.hg_last_error()
+
+
+def test_backward_validates_before_touching_the_gpu():
+    lib = _lib.lib()
+    s = _lib.RasterInputs()
+    s.P, s.N, s.W, s.H = 4, 4, 32, 32
+    bwd = lambda: lib.hg_raster_backward(ctypes.byref(s), 0, *([None] * 21), None)  # noqa: E731
+    # every pointer is checked before the first CUDA call (fake non-null pointers are never dereferenced)
+    assert bwd() == 1 and b"mandatory pointer" in lib.hg_last_error()
+    for f in ("means3D", "opacities", "background", "viewmatrix", "projmatrix", "campos", "shs", "scales"):
+        setattr(s, f, 256)
+    s.M, s.D = 16, 3
+    assert bwd() == 1 and b"scale/rotation pair" in lib.hg_last_error()
+    s.rotations = 260
+    assert bwd() == 1 and b"rotations must be 16-byte aligned" in lib.hg_last_error()
+    # the same arguments with an aligned rotations pointer pass validate() and stop at the missing outputs
+    s.rotations = 272
+    assert bwd() == 1 and b"hg_raster_backward: a mandatory pointer is NULL" in lib.hg_last_error()
+    s.rotations = 264
+    rc = lib.hg_raster_backward_chunked(ctypes.byref(s), 0, *([None] * 21), 1, _lib.CHUNK_FN(0), None, None, 0.0, None,
+                                        0, None)
+    assert rc == 1 and b"rotations must be 16-byte aligned" in lib.hg_last_error()
 
 
 def test_python_api_surface_matches_reference():

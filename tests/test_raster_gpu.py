@@ -456,8 +456,11 @@ def test_sh_gradient_sink_and_chunked_backward(cuda_device):
         ru.OUR_C.rasterize_gaussians_backward(*bh, sh_sink=(torch.zeros(hier["means3D"].shape[0], 16, 3, device=dev), 0.0))
 
 
-@pytest.mark.parametrize("degree", [3, 1])
-def test_sh_gradient_factors_rebuild_the_summed_rows(cuda_device, degree):
+# (degree, SH coefficients M): rows of 3 M floats that are not a multiple of 4 take the per-thread paths of both kernels
+@pytest.mark.parametrize("degree,M", [pytest.param(3, 16, id="3"), pytest.param(1, 16, id="1"),
+                                      pytest.param(0, 1, id="0-M1"), pytest.param(1, 9, id="1-M9"),
+                                      pytest.param(2, 15, id="2-M15")])
+def test_sh_gradient_factors_rebuild_the_summed_rows(cuda_device, degree, M):
     """Factored exchange (include/hidegs_exchange.h): with `sh_factor` the backward writes three colour-gradient factors
     per Gaussian + the camera centre instead of the SH rows; hg_sh_gradient_from_factors over the blocks of several
     views rebuilds exactly the sum of the rows the plain backward writes for those views; every other gradient is
@@ -471,7 +474,7 @@ def test_sh_gradient_factors_rebuild_the_summed_rows(cuda_device, degree):
     want = None
     some_dead = False
     for v, eye in enumerate(eyes):
-        case = ru.build_case(N, W, H, seed=21, sh_degree=degree, eye=eye)
+        case = ru.build_case(N, W, H, seed=21, sh_degree=degree, eye=eye, sh_coeffs=M)
         fa = ru.op_args(case, dev)
         fwd = ru.OUR_C.rasterize_gaussians(*fa)
         ba = ru.bwd_args(fa, fwd, syn.upstream_grads(W, H, seed=v), dev)
