@@ -8,7 +8,8 @@ EXPORTED_SYMBOLS = (
     "hg_normal_consistency_workspace_bytes", "hg_normal_consistency_loss", "hg_adam_step", "hg_densification_stats", "hg_expand_to_size_workspace_bytes", "hg_expand_to_size",
     "hg_interpolation_weights", "hg_hier_interpolate", "hg_hier_interpolate_backward",
     "hg_dist2_knn3_workspace_bytes", "hg_dist2_knn3", "hg_densify_workspace_bytes", "hg_densify_plan", "hg_densify_apply",
-    "hg_reset_opacity",
+    "hg_reset_opacity", "hg_camera_pose_apply", "hg_camera_pose_workspace_bytes", "hg_prologue_backward_pose",
+    "hg_camera_pose_grad_finish",
 )
 
 
@@ -52,6 +53,11 @@ def lib():
         "hg_densify_plan": (ci, [vp, p64, i64, vp, i32, f64, f64, f64, f64, f64, vp, p64, p64, p64, p64, vp]),
         "hg_densify_apply": (ci, [vp, vp, vp, p64, i64, vp, vp, vp, p64, i64, vp, ctypes.c_uint64, vp, vp]),
         "hg_reset_opacity": (ci, [vp, vp, vp, i64, vp]),
+        "hg_camera_pose_apply": (ci, [vp, vp, vp, vp, i32, i32, vp, vp]),
+        "hg_camera_pose_workspace_bytes": (sz, [i64]),
+        "hg_prologue_backward_pose": (ci, [vp, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f32, vp,
+                                           vp, vp, vp, vp, vp, vp]),
+        "hg_camera_pose_grad_finish": (ci, [vp, i32, i32, i64, vp, vp, vp, vp]),
     }
     for name, (res, args) in proto.items():
         fn = getattr(L, name)

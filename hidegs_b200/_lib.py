@@ -44,7 +44,7 @@ class RasterLayout(ctypes.Structure):
 # Every symbol include/hidegs_raster.h declares (checked by the CPU test-suite).
 EXPORTED_SYMBOLS = (
     "hg_raster_layout_query", "hg_raster_forward", "hg_raster_backward_accum_bytes", "hg_raster_backward",
-    "hg_raster_backward_chunked",
+    "hg_raster_backward_chunked", "hg_raster_backward_pose",
     "hg_mark_visible", "hg_raster_debug_keys", "hg_launch_count", "hg_reset_launch_count", "hg_last_error", "hg_version",
     "hg_profile_enable", "hg_profile_collect",
 )
@@ -77,6 +77,8 @@ def lib():
     L.hg_raster_backward.restype = ctypes.c_int
     L.hg_raster_backward_chunked.argtypes = L.hg_raster_backward.argtypes[:-1] + [i32, CHUNK_FN, vp, vp, ctypes.c_float, vp, i32, vp]
     L.hg_raster_backward_chunked.restype = ctypes.c_int
+    L.hg_raster_backward_pose.argtypes = L.hg_raster_backward_chunked.argtypes[:-1] + [vp, vp]
+    L.hg_raster_backward_pose.restype = ctypes.c_int
     L.hg_raster_debug_keys.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]
     L.hg_raster_debug_keys.restype = ctypes.c_int
     L.hg_mark_visible.argtypes = [i32, vp, vp, vp, vp, vp]

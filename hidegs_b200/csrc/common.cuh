@@ -155,7 +155,22 @@ int launch_preprocess_bwd(const hg_raster_inputs& in, const GeomState& g, const 
                           float* dL_dcov3D, float* dL_dsh, float* dL_dscales,
                           float* dL_drotations, float* dL_dall_map, cudaStream_t stream, int slot_begin = 0,
                           int slot_end = -1, float* sh_sink = nullptr, float sh_beta = 0.f,
-                          float* sh_factor = nullptr, bool skip_culled_rows = false);
+                          float* sh_factor = nullptr, bool skip_culled_rows = false,
+                          double* pose_partial = nullptr);
+// Camera pose gradient partials (camera_pose.cu): one row of kPosePartialStride doubles ([0..2] dL/drho, [3..5] the
+// torque) per CTA of the pose variants of the per-Gaussian backward (128-slot CTAs) and of the prologue backward
+// (256-row CTAs).  The CTA counts depend on the Gaussian count only.
+constexpr int kPosePartialStride = 8;
+constexpr int kPoseRasterSlots = 128;
+constexpr int kPosePrologueRows = 256;
+// pose workspace of N Gaussians: [rasterizer partials | prologue partials], each part 256-byte aligned
+static inline size_t camera_pose_prologue_offset(int64_t N) {
+  return align_up((size_t)((N + kPoseRasterSlots - 1) / kPoseRasterSlots) * kPosePartialStride * sizeof(double), 256);
+}
+static inline size_t camera_pose_workspace_bytes(int64_t N) {
+  return camera_pose_prologue_offset(N) +
+         align_up((size_t)((N + kPosePrologueRows - 1) / kPosePrologueRows) * kPosePartialStride * sizeof(double), 256);
+}
 int launch_sh_from_factors(int N, int D, int M, int n_views, const float* means3D, const float* factors,
                            size_t view_stride, float* dL_dsh, float beta, cudaStream_t stream);
 int preprocess_bwd_block_slots();

@@ -10,6 +10,7 @@
 #include "reduce.cuh"
 #include "../../include/hidegs_geometry.h"
 
+#include <climits>
 #include <cmath>
 
 namespace hg {
@@ -45,11 +46,13 @@ __device__ __forceinline__ int argmin3(float a, float b, float c) {
 }
 
 // One row of input_all_map and (BACKWARD) of its gradient: `m` = index of the smallest scaling axis, `q` the rotation as
-// the renderer sees it (activated).  out5 / g5 point at the row's five floats.
-template <bool BACKWARD>
+// the renderer sees it (activated).  out5 / g5 point at the row's five floats.  POSE: the camera side of the row's
+// gradient is added to pose[0..5]: dL/drho = g4 n_cam, and the torque n_cam x dL/dn_cam + p_cam x dL/dp_cam, in which
+// the two terms of d = n_cam . p_cam cancel (d does not change when the camera turns), leaving n_cam x g5[0..2].
+template <bool BACKWARD, bool POSE = false>
 __device__ __forceinline__ void all_map_row(const View& V, const float px, const float py, const float pz, const int m,
                                             const float4 q, float* __restrict__ out5, const float* __restrict__ g5,
-                                            float (&dxyz)[3], float4& drot) {
+                                            float (&dxyz)[3], float4& drot, float* pose = nullptr) {
   const float qq = q.x * q.x + q.y * q.y + q.z * q.z + q.w * q.w;
   const float s = 2.0f / qq;
   float col[3];
@@ -75,6 +78,12 @@ __device__ __forceinline__ void all_map_row(const View& V, const float px, const
   for (int j = 0; j < 3; ++j) {
     dln[j] = g5[j] + g4 * pc[j];
     dpc[j] = g4 * ln[j];
+  }
+  if constexpr (POSE) {
+    pose[0] += dpc[0]; pose[1] += dpc[1]; pose[2] += dpc[2];
+    pose[3] += ln[1] * g5[2] - ln[2] * g5[1];
+    pose[4] += ln[2] * g5[0] - ln[0] * g5[2];
+    pose[5] += ln[0] * g5[1] - ln[1] * g5[0];
   }
   float dn[3];
 #pragma unroll
@@ -206,17 +215,16 @@ activate_bwd_kernel(const float* __restrict__ rs, const float* __restrict__ rr, 
 // skipped (beta = 1) or zero-filled (beta = 0) without reading their gradient rows — which the rasterizer's backward
 // therefore need not write (HG_BWD_SKIP_CULLED_ROWS).  Replaces all_map_kernel<true>, two adds, one addcmul and
 // activate_bwd_kernel (five passes over N rows) of the executor.
-__global__ void __launch_bounds__(256)
-prologue_bwd_kernel(const float* __restrict__ rs, const float* __restrict__ rr, const float* __restrict__ ro,
-                    const float* __restrict__ xyz, const int64_t N, const int* __restrict__ radii,
-                    const float* __restrict__ viewmatrix, const float* __restrict__ campos,
-                    const float* __restrict__ g_xyz, const float* __restrict__ g_o, const float* __restrict__ g_s,
-                    const float* __restrict__ g_r, const float* __restrict__ g_all_map,
-                    const float* __restrict__ g_s_extra, const float* __restrict__ extra_scale, const float beta,
-                    float* __restrict__ d_xyz, float* __restrict__ d_o, float* __restrict__ d_s,
-                    float* __restrict__ d_r) {
-  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= N) return;
+template <bool POSE>
+__device__ __forceinline__ void
+prologue_bwd_row(const int64_t n, const float* __restrict__ rs, const float* __restrict__ rr, const float* __restrict__ ro,
+                 const float* __restrict__ xyz, const int* __restrict__ radii,
+                 const float* __restrict__ viewmatrix, const float* __restrict__ campos,
+                 const float* __restrict__ g_xyz, const float* __restrict__ g_o, const float* __restrict__ g_s,
+                 const float* __restrict__ g_r, const float* __restrict__ g_all_map,
+                 const float* __restrict__ g_s_extra, const float* __restrict__ extra_scale, const float beta,
+                 float* __restrict__ d_xyz, float* __restrict__ d_o, float* __restrict__ d_s,
+                 float* __restrict__ d_r, float* pose) {
   const bool acc = beta != 0.0f;
   float4* const dst_r = reinterpret_cast<float4*>(d_r) + n;
   if (radii && radii[n] <= 0) {
@@ -246,8 +254,8 @@ prologue_bwd_kernel(const float* __restrict__ rs, const float* __restrict__ rr, 
     for (int i = 0; i < 3; ++i) V.cam[i] = __ldg(campos + i);
     float dxyz[3];
     float4 drot;
-    all_map_row<true>(V, xyz[3 * n], xyz[3 * n + 1], xyz[3 * n + 2], argmin3(e[0], e[1], e[2]), y, nullptr,
-                      g_all_map + 5 * n, dxyz, drot);
+    all_map_row<true, POSE>(V, xyz[3 * n], xyz[3 * n + 1], xyz[3 * n + 2], argmin3(e[0], e[1], e[2]), y, nullptr,
+                            g_all_map + 5 * n, dxyz, drot, pose);
     gx[0] += dxyz[0]; gx[1] += dxyz[1]; gx[2] += dxyz[2];
     g = make_float4(g.x + drot.x, g.y + drot.y, g.z + drot.z, g.w + drot.w);
   }
@@ -278,6 +286,41 @@ prologue_bwd_kernel(const float* __restrict__ rs, const float* __restrict__ rr, 
       d = make_float4(p.x + d.x, p.y + d.y, p.z + d.z, p.w + d.w);
     }
     *dst_r = d;
+  }
+}
+
+// POSE: the rows' camera-side all_map gradients (all_map_row) summed over the CTA in double in a fixed order (warp
+// butterflies, then the 8 warps in index order) -> pose_partial[blockIdx.x][0..5]; the grid depends on N only.
+template <bool POSE>
+__global__ void __launch_bounds__(kPosePrologueRows)
+prologue_bwd_kernel(const float* __restrict__ rs, const float* __restrict__ rr, const float* __restrict__ ro,
+                    const float* __restrict__ xyz, const int64_t N, const int* __restrict__ radii,
+                    const float* __restrict__ viewmatrix, const float* __restrict__ campos,
+                    const float* __restrict__ g_xyz, const float* __restrict__ g_o, const float* __restrict__ g_s,
+                    const float* __restrict__ g_r, const float* __restrict__ g_all_map,
+                    const float* __restrict__ g_s_extra, const float* __restrict__ extra_scale, const float beta,
+                    float* __restrict__ d_xyz, float* __restrict__ d_o, float* __restrict__ d_s,
+                    float* __restrict__ d_r, double* __restrict__ pose_partial) {
+  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  float pose[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (n < N)
+    prologue_bwd_row<POSE>(n, rs, rr, ro, xyz, radii, viewmatrix, campos, g_xyz, g_o, g_s, g_r, g_all_map, g_s_extra,
+                           extra_scale, beta, d_xyz, d_o, d_s, d_r, pose);
+  if constexpr (POSE) {
+    __shared__ double s_pose[kPosePrologueRows / 32][6];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+      const double w = warp_sum_double((double)pose[k]);
+      if (lane == 0) s_pose[warp][k] = w;
+    }
+    __syncthreads();
+    if (threadIdx.x < 6) {
+      double a = 0.0;
+#pragma unroll
+      for (int w = 0; w < kPosePrologueRows / 32; ++w) a += s_pose[w][threadIdx.x];
+      pose_partial[(size_t)blockIdx.x * kPosePartialStride + threadIdx.x] = a;
+    }
   }
 }
 
@@ -668,12 +711,20 @@ int hg_activate_params_backward(const float* raw_scaling, const float* raw_rotat
   return HG_OK;
 }
 
-int hg_prologue_backward(const float* raw_scaling, const float* raw_rotation, const float* raw_opacity, const float* xyz,
-                         int64_t N, int32_t F, const int32_t* radii, const float* viewmatrix, const float* campos,
-                         const float* g_xyz, const float* g_features, const float* g_opacity, const float* g_scaling,
-                         const float* g_rotation, const float* g_all_map, const float* g_scaling_extra,
-                         const float* extra_scale, float beta, float* d_xyz, float* d_features, float* d_opacity,
-                         float* d_scaling, float* d_rotation, void* st_) {
+}  // extern "C"
+
+// hg_prologue_backward and hg_prologue_backward_pose: pose_workspace == NULL is the plain prologue backward.
+static int prologue_backward_impl(const float* raw_scaling, const float* raw_rotation, const float* raw_opacity,
+                                  const float* xyz, int64_t N, int32_t F, const int32_t* radii, const float* viewmatrix,
+                                  const float* campos, const float* g_xyz, const float* g_features,
+                                  const float* g_opacity, const float* g_scaling, const float* g_rotation,
+                                  const float* g_all_map, const float* g_scaling_extra, const float* extra_scale,
+                                  float beta, float* d_xyz, float* d_features, float* d_opacity, float* d_scaling,
+                                  float* d_rotation, void* pose_workspace, void* st_) {
+  if (pose_workspace && (N > INT32_MAX || (reinterpret_cast<uintptr_t>(pose_workspace) & 15))) {
+    set_error("hg_prologue_backward_pose: bad argument (N must fit int32, the workspace must be 16-byte aligned)");
+    return HG_ERR_INVALID_ARG;
+  }
   if (N < 0 || F < 0 || !(beta == 0.0f || beta == 1.0f) ||
       (N > 0 && (!raw_scaling || !raw_rotation || !raw_opacity || !d_xyz || !d_opacity || !d_scaling || !d_rotation ||
                  (g_all_map && (!xyz || !viewmatrix || !campos)) || (F > 0 && g_features && !d_features))) ||
@@ -684,16 +735,47 @@ int hg_prologue_backward(const float* raw_scaling, const float* raw_rotation, co
   }
   if (N == 0) return HG_OK;
   cudaStream_t st = (cudaStream_t)st_;
-  prologue_bwd_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(raw_scaling, raw_rotation, raw_opacity, xyz, N, radii,
-                                                                     viewmatrix, campos, g_xyz, g_opacity, g_scaling,
-                                                                     g_rotation, g_all_map, g_scaling_extra, extra_scale,
-                                                                     beta, d_xyz, d_opacity, d_scaling, d_rotation);
-  HG_POST_LAUNCH(false, st, "prologue_bwd");
+  double* const pose_partial = static_cast<double*>(pose_workspace);
+  auto kernel = pose_partial ? prologue_bwd_kernel<true> : prologue_bwd_kernel<false>;
+  kernel<<<(unsigned)((N + kPosePrologueRows - 1) / kPosePrologueRows), kPosePrologueRows, 0, st>>>(
+      raw_scaling, raw_rotation, raw_opacity, xyz, N, radii, viewmatrix, campos, g_xyz, g_opacity, g_scaling, g_rotation,
+      g_all_map, g_scaling_extra, extra_scale, beta, d_xyz, d_opacity, d_scaling, d_rotation, pose_partial);
+  HG_POST_LAUNCH(false, st, pose_partial ? "prologue_bwd_pose" : "prologue_bwd");
   if (F > 0 && g_features) {  // NULL: the feature gradient already sits in d_features (rasterizer SH sink)
     axpby4_kernel<<<148 * 8, 256, 0, st>>>((const float4*)g_features, N * (int64_t)F / 4, beta, (float4*)d_features);
     HG_POST_LAUNCH(false, st, "features_grad_accumulate");
   }
   return HG_OK;
+}
+
+extern "C" {
+
+int hg_prologue_backward(const float* raw_scaling, const float* raw_rotation, const float* raw_opacity, const float* xyz,
+                         int64_t N, int32_t F, const int32_t* radii, const float* viewmatrix, const float* campos,
+                         const float* g_xyz, const float* g_features, const float* g_opacity, const float* g_scaling,
+                         const float* g_rotation, const float* g_all_map, const float* g_scaling_extra,
+                         const float* extra_scale, float beta, float* d_xyz, float* d_features, float* d_opacity,
+                         float* d_scaling, float* d_rotation, void* st_) {
+  return prologue_backward_impl(raw_scaling, raw_rotation, raw_opacity, xyz, N, F, radii, viewmatrix, campos, g_xyz,
+                                g_features, g_opacity, g_scaling, g_rotation, g_all_map, g_scaling_extra, extra_scale,
+                                beta, d_xyz, d_features, d_opacity, d_scaling, d_rotation, nullptr, st_);
+}
+
+int hg_prologue_backward_pose(const float* raw_scaling, const float* raw_rotation, const float* raw_opacity,
+                              const float* xyz, int64_t N, int32_t F, const int32_t* radii, const float* viewmatrix,
+                              const float* campos, const float* g_xyz, const float* g_features, const float* g_opacity,
+                              const float* g_scaling, const float* g_rotation, const float* g_all_map,
+                              const float* g_scaling_extra, const float* extra_scale, float beta, float* d_xyz,
+                              float* d_features, float* d_opacity, float* d_scaling, float* d_rotation,
+                              void* pose_workspace, void* st_) {
+  if (!pose_workspace) {
+    set_error("hg_prologue_backward_pose: pose_workspace is NULL");
+    return HG_ERR_INVALID_ARG;
+  }
+  return prologue_backward_impl(raw_scaling, raw_rotation, raw_opacity, xyz, N, F, radii, viewmatrix, campos, g_xyz,
+                                g_features, g_opacity, g_scaling, g_rotation, g_all_map, g_scaling_extra, extra_scale,
+                                beta, d_xyz, d_features, d_opacity, d_scaling, d_rotation,
+                                static_cast<char*>(pose_workspace) + camera_pose_prologue_offset(N), st_);
 }
 
 int hg_depth_normal(const float* plane_depth, const float* alpha, int32_t H, int32_t W, hg_intrinsics K,

@@ -16,13 +16,14 @@
 // gradients are zeroed and (1-t) x mean gradient is pushed to the parent
 // (backward.cu:459-495).
 #include "common.cuh"
+#include "reduce.cuh"
 #include "sh_stage.cuh"
 
 namespace hg {
 
 namespace {
 
-constexpr int kThreads = 128;
+constexpr int kThreads = kPoseRasterSlots;
 constexpr int kWarps = kThreads / 32;
 constexpr int kShStrideMax = 48 + 1;  // M <= 16 coefficients x 3 channels, odd stride
 
@@ -38,6 +39,11 @@ __device__ __forceinline__ void store_or_add3(float* dst, float a, float b, floa
   }
 }
 
+// POSE (camera pose refinement, DESIGN.md §3): every rendered slot also forms the camera side of its gradient — the
+// gradient g_p w.r.t. its camera-frame mean over every path, and the torque p_cam x g_p(non-SH) + vee(G - G^T) with
+// G = dL/dW W^T of the covariance path (the SH view direction moves with the camera centre, i.e. with rho only) — and
+// the CTA writes the sum of these six numbers (double, fixed order) to pose_partial[global block][0..5].
+template <bool POSE>
 __global__ void __launch_bounds__(kThreads)
 preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, const int* __restrict__ indices,
                       const int* __restrict__ parent_indices, const float* __restrict__ ts,
@@ -56,7 +62,8 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
                       float* __restrict__ dL_dmeans3D, float* __restrict__ dL_dcov3D,
                       float* __restrict__ dL_dsh, float* __restrict__ dL_dscales,
                       float* __restrict__ dL_drotations, float* __restrict__ dL_dall_map,
-                      float* __restrict__ sh_sink, const float sh_beta, float* __restrict__ sh_factor) {
+                      float* __restrict__ sh_sink, const float sh_beta, float* __restrict__ sh_factor,
+                      double* __restrict__ pose_partial) {
   // SH rows (read AND written, 2 x 192 B per Gaussian at degree 3: 60 % of this kernel's traffic) move through a
   // per-warp shared-memory tile with coalesced 128-bit accesses when the warp's rows are contiguous (no index
   // remap); each thread then works on its own row of the tile.
@@ -98,6 +105,8 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
     else stage_sh_rows<0>(shs, warp_base, sh_total, row, lane, tile, alive_mask);
     __syncwarp();
   }
+  // camera side of this slot's gradient (POSE): [0..2] dL/drho, [3..5] torque; zero for culled slots
+  float pose[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   do {  // single-trip block: `break` = this thread is done (it still joins the cooperative store below)
   if (!in_range) break;
   const int idx = indices ? __ldg(indices + t_idx) : t_idx;
@@ -160,6 +169,7 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
 
   float tx = v[0] * mx + v[4] * my + v[8] * mz + v[12];
   float ty = v[1] * mx + v[5] * my + v[9] * mz + v[13];
+  const float pcx = tx, pcy = ty;  // (POSE) the camera-frame mean before the frustum clamp
   const float tz = v[2] * mx + v[6] * my + v[10] * mz + v[14];
   const float limx = 1.3f * tan_fovx, limy = 1.3f * tan_fovy;
   const float txtz = tx / tz, tytz = ty / tz;
@@ -247,6 +257,14 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
   float dtz = -h_x * itz2 * dJ00 - h_y * itz2 * dJ11 + (2.f * h_x * tx) * itz3 * dJ02 +
               (2.f * h_y * ty) * itz3 * dJ12;
   if (has_invdepth) dtz -= dinvd / (tz * tz);
+  if constexpr (POSE) {
+    // torque of the covariance path: G = J^T A, A = dL/dT W^T (2 x 3; A00, A02, A11, A12 are the dJ above)
+    const float A01 = v[1] * dT00 + v[5] * dT01 + v[9] * dT02;
+    const float A10 = v[0] * dT10 + v[4] * dT11 + v[8] * dT12;
+    pose[3] = (J02 * A01 + J12 * dJ11) - J11 * dJ12;  // G21 - G12
+    pose[4] = J00 * dJ02 - (J02 * dJ00 + J12 * A10);  // G02 - G20
+    pose[5] = J11 * A10 - J00 * A01;                  // G10 - G01
+  }
   float dmean_x = v[0] * dtx + v[1] * dty + v[2] * dtz;
   float dmean_y = v[4] * dtx + v[5] * dty + v[6] * dtz;
   float dmean_z = v[8] * dtx + v[9] * dty + v[10] * dtz;
@@ -260,6 +278,15 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
     dmean_x += (pm[0] * m_w - pm[3] * mul1) * dm2x + (pm[1] * m_w - pm[3] * mul2) * dm2y;
     dmean_y += (pm[4] * m_w - pm[7] * mul1) * dm2x + (pm[5] * m_w - pm[7] * mul2) * dm2y;
     dmean_z += (pm[8] * m_w - pm[11] * mul1) * dm2x + (pm[9] * m_w - pm[11] * mul2) * dm2y;
+  }
+
+  if constexpr (POSE) {  // + p_cam x g_p over every path but the SH view direction (g_p = W dL/dmean)
+    const float gx = v[0] * dmean_x + v[4] * dmean_y + v[8] * dmean_z;
+    const float gy = v[1] * dmean_x + v[5] * dmean_y + v[9] * dmean_z;
+    const float gz = v[2] * dmean_x + v[6] * dmean_y + v[10] * dmean_z;
+    pose[3] += pcy * gz - tz * gy;
+    pose[4] += tz * gx - pcx * gz;
+    pose[5] += pcx * gy - pcy * gx;
   }
 
   // Parent handling decides what survives (backward.cu:459-495).
@@ -395,6 +422,12 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
                  y * Dr[1][2] + x * Dr[2][0] + y * Dr[2][1]);
   }
 
+  if constexpr (POSE) {  // dL/drho = W dL/dmean over every path (the camera centre moves by -R^T rho)
+    pose[0] = v[0] * dmean_x + v[4] * dmean_y + v[8] * dmean_z;
+    pose[1] = v[1] * dmean_x + v[5] * dmean_y + v[9] * dmean_z;
+    pose[2] = v[2] * dmean_x + v[6] * dmean_y + v[10] * dmean_z;
+  }
+
   if (has_parent) {
     const float t = __ldg(ts + t_idx);
     dopac = 0.f;
@@ -429,6 +462,21 @@ preprocess_bwd_kernel(const int P, const int block0, const int D, const int M, c
   } else if (staged && (alive_mask || !prezeroed)) {
     __syncwarp();
     unstage_sh_rows(dL_dsh, warp_base, sh_total, row, lane, tile, alive_mask, !prezeroed);
+  }
+  if constexpr (POSE) {  // warp butterflies in double, then the 4 warps in index order: bits fixed by the slot count
+    __shared__ double s_pose[kWarps][6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+      const double w = warp_sum_double((double)pose[k]);
+      if (lane == 0) s_pose[warp][k] = w;
+    }
+    __syncthreads();
+    if (threadIdx.x < 6) {
+      double acc = 0.0;
+#pragma unroll
+      for (int w = 0; w < kWarps; ++w) acc += s_pose[w][threadIdx.x];
+      pose_partial[(size_t)(blockIdx.x + block0) * kPosePartialStride + threadIdx.x] = acc;
+    }
   }
 }
 
@@ -529,7 +577,8 @@ int launch_preprocess_bwd(const hg_raster_inputs& in, const GeomState& g, const 
                           float* dL_dcolors, float* dL_dinvdepths, float* dL_dmeans3D,
                           float* dL_dcov3D, float* dL_dsh, float* dL_dscales,
                           float* dL_drotations, float* dL_dall_map, cudaStream_t stream, int slot_begin,
-                          int slot_end, float* sh_sink, float sh_beta, float* sh_factor, bool skip_culled_rows) {
+                          int slot_end, float* sh_sink, float sh_beta, float* sh_factor, bool skip_culled_rows,
+                          double* pose_partial) {
   // "prezeroed": the kernel leaves the rows of culled slots alone — because the caller zero-filled the arrays (index
   // remap / parents: rows are scattered and accumulated), or because it never reads them (HG_BWD_SKIP_CULLED_ROWS)
   const bool prezeroed = in.indices != nullptr || in.parent_indices != nullptr || skip_culled_rows;
@@ -548,17 +597,22 @@ int launch_preprocess_bwd(const hg_raster_inputs& in, const GeomState& g, const 
     set_error("preprocess_bwd: SH gradient factors need SH input, no index remap and no SH sink");
     return HG_ERR_INVALID_ARG;
   }
+  if (pose_partial && (in.indices || in.parent_indices)) {
+    set_error("preprocess_bwd: the camera pose gradient needs contiguous slots (no render or parent indices)");
+    return HG_ERR_INVALID_ARG;
+  }
   if (slot_begin % kThreads != 0 || slot_begin >= slot_end) {
     set_error("preprocess_bwd: bad slot range [%d, %d)", slot_begin, slot_end);
     return HG_ERR_INVALID_ARG;
   }
-  preprocess_bwd_kernel<<<(slot_end - slot_begin + kThreads - 1) / kThreads, kThreads, 0, stream>>>(
+  auto kernel = pose_partial ? preprocess_bwd_kernel<true> : preprocess_bwd_kernel<false>;
+  kernel<<<(slot_end - slot_begin + kThreads - 1) / kThreads, kThreads, 0, stream>>>(
       slot_end, slot_begin / kThreads, in.D, in.M, in.indices, in.parent_indices, in.ts, in.means3D, radii, in.shs, g.clamped,
       in.opacities, in.scales, in.rotations, in.scale_modifier, cov, in.cov3D_precomp != nullptr,
       in.viewmatrix, in.projmatrix, in.campos, focal_x, focal_y, in.tan_fovx, in.tan_fovy, accum,
       has_invdepth, prezeroed, dL_dmeans2D, dL_dconic, dL_dopacity, dL_dcolors, dL_dinvdepths,
-      dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales, dL_drotations, dL_dall_map, sh_sink, sh_beta, sh_factor);
-  HG_POST_LAUNCH(in.debug, stream, "preprocess_bwd");
+      dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales, dL_drotations, dL_dall_map, sh_sink, sh_beta, sh_factor, pose_partial);
+  HG_POST_LAUNCH(in.debug, stream, pose_partial ? "preprocess_bwd_pose" : "preprocess_bwd");
   return HG_OK;
 }
 

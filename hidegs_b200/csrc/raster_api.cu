@@ -285,19 +285,27 @@ int hg_raster_backward(const hg_raster_inputs* in, int32_t R, const int32_t* rad
                                     dL_drotations, dL_dall_map, 1, nullptr, nullptr, nullptr, 0.f, nullptr, 0, stream_);
 }
 
-int hg_raster_backward_chunked(const hg_raster_inputs* in, int32_t R, const int32_t* radii,
-                               const char* geom_buffer, const char* binning_buffer,
-                               const char* image_buffer, const float* all_map_pixels,
-                               const float* dL_dpix, const float* dL_dout_all_map,
-                               const float* dL_dout_plane_depth, const float* dL_dout_invdepth,
-                               char* accum, float* dL_dmeans2D, float* dL_dconic, float* dL_dopacity,
-                               float* dL_dcolors, float* dL_dinvdepths, float* dL_dmeans3D,
-                               float* dL_dcov3D, float* dL_dsh, float* dL_dscales, float* dL_drotations,
-                               float* dL_dall_map, int32_t n_chunks, hg_chunk_fn on_chunk, void* chunk_ctx,
-                               float* sh_sink, float sh_beta, float* sh_factor, int32_t flags, void* stream_) {
+}  // extern "C"
+
+// hg_raster_backward_chunked and hg_raster_backward_pose: pose_workspace == NULL is the plain backward.
+static int raster_backward_impl(const hg_raster_inputs* in, int32_t R, const int32_t* radii, const char* geom_buffer,
+                                const char* binning_buffer, const char* image_buffer, const float* all_map_pixels,
+                                const float* dL_dpix, const float* dL_dout_all_map, const float* dL_dout_plane_depth,
+                                const float* dL_dout_invdepth, char* accum, float* dL_dmeans2D, float* dL_dconic,
+                                float* dL_dopacity, float* dL_dcolors, float* dL_dinvdepths, float* dL_dmeans3D,
+                                float* dL_dcov3D, float* dL_dsh, float* dL_dscales, float* dL_drotations,
+                                float* dL_dall_map, int32_t n_chunks, hg_chunk_fn on_chunk, void* chunk_ctx,
+                                float* sh_sink, float sh_beta, float* sh_factor, int32_t flags, void* pose_workspace,
+                                void* stream_) {
   g_err[0] = 0;
   int rc = validate(in);
   if (rc) return rc;
+  if (pose_workspace && (in->indices || in->parent_indices || in->N != in->P ||
+                         (reinterpret_cast<uintptr_t>(pose_workspace) & 15))) {
+    set_error("hg_raster_backward_pose: the camera pose gradient needs every Gaussian as one slot (no render or parent "
+              "indices, P == N) and a 16-byte aligned workspace");
+    return HG_ERR_INVALID_ARG;
+  }
   if (in->P == 0) return HG_OK;
   if (!radii || !geom_buffer || !image_buffer || !dL_dpix || !accum || !dL_dmeans2D ||
       !dL_dopacity || !dL_dcolors || !dL_dmeans3D || !dL_dcov3D || (in->shs && !dL_dsh) || !dL_dscales ||
@@ -348,11 +356,53 @@ int hg_raster_backward_chunked(const hg_raster_inputs* in, int32_t R, const int3
                                dL_dmeans2D, dL_dconic, dL_dopacity, dL_dcolors, dL_dinvdepths,
                                dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales, dL_drotations,
                                dL_dall_map, stream, p0, p1, sh_sink, sh_beta, sh_factor,
-                               (flags & HG_BWD_SKIP_CULLED_ROWS) != 0);
+                               (flags & HG_BWD_SKIP_CULLED_ROWS) != 0, static_cast<double*>(pose_workspace));
     if (rc) return rc;
     if (on_chunk) on_chunk(chunk_ctx, chunk, p0, p1, stream_);
   }
   return HG_OK;
+}
+
+extern "C" {
+
+int hg_raster_backward_chunked(const hg_raster_inputs* in, int32_t R, const int32_t* radii,
+                               const char* geom_buffer, const char* binning_buffer,
+                               const char* image_buffer, const float* all_map_pixels,
+                               const float* dL_dpix, const float* dL_dout_all_map,
+                               const float* dL_dout_plane_depth, const float* dL_dout_invdepth,
+                               char* accum, float* dL_dmeans2D, float* dL_dconic, float* dL_dopacity,
+                               float* dL_dcolors, float* dL_dinvdepths, float* dL_dmeans3D,
+                               float* dL_dcov3D, float* dL_dsh, float* dL_dscales, float* dL_drotations,
+                               float* dL_dall_map, int32_t n_chunks, hg_chunk_fn on_chunk, void* chunk_ctx,
+                               float* sh_sink, float sh_beta, float* sh_factor, int32_t flags, void* stream_) {
+  return raster_backward_impl(in, R, radii, geom_buffer, binning_buffer, image_buffer, all_map_pixels, dL_dpix,
+                              dL_dout_all_map, dL_dout_plane_depth, dL_dout_invdepth, accum, dL_dmeans2D, dL_dconic,
+                              dL_dopacity, dL_dcolors, dL_dinvdepths, dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales,
+                              dL_drotations, dL_dall_map, n_chunks, on_chunk, chunk_ctx, sh_sink, sh_beta, sh_factor,
+                              flags, nullptr, stream_);
+}
+
+int hg_raster_backward_pose(const hg_raster_inputs* in, int32_t R, const int32_t* radii,
+                            const char* geom_buffer, const char* binning_buffer,
+                            const char* image_buffer, const float* all_map_pixels,
+                            const float* dL_dpix, const float* dL_dout_all_map,
+                            const float* dL_dout_plane_depth, const float* dL_dout_invdepth,
+                            char* accum, float* dL_dmeans2D, float* dL_dconic, float* dL_dopacity,
+                            float* dL_dcolors, float* dL_dinvdepths, float* dL_dmeans3D,
+                            float* dL_dcov3D, float* dL_dsh, float* dL_dscales, float* dL_drotations,
+                            float* dL_dall_map, int32_t n_chunks, hg_chunk_fn on_chunk, void* chunk_ctx,
+                            float* sh_sink, float sh_beta, float* sh_factor, int32_t flags, void* pose_workspace,
+                            void* stream_) {
+  if (!pose_workspace) {
+    g_err[0] = 0;
+    set_error("hg_raster_backward_pose: pose_workspace is NULL");
+    return HG_ERR_INVALID_ARG;
+  }
+  return raster_backward_impl(in, R, radii, geom_buffer, binning_buffer, image_buffer, all_map_pixels, dL_dpix,
+                              dL_dout_all_map, dL_dout_plane_depth, dL_dout_invdepth, accum, dL_dmeans2D, dL_dconic,
+                              dL_dopacity, dL_dcolors, dL_dinvdepths, dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales,
+                              dL_drotations, dL_dall_map, n_chunks, on_chunk, chunk_ctx, sh_sink, sh_beta, sh_factor,
+                              flags, pose_workspace, stream_);
 }
 
 int hg_raster_debug_keys(int32_t P, int32_t W, int32_t H, int32_t R, const int32_t* radii, const char* geom_buffer,

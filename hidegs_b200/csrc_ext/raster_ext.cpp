@@ -16,6 +16,7 @@
 //   sh_factor           write the three colour-gradient factors per Gaussian instead of the SH rows (factored exchange)
 //   grad_arena          caller-owned flat fp32 tensor the gradients are written into (e.g. multicast symmetric memory)
 //   n_chunks/chunk_hook issue the per-Gaussian backward in slot ranges and call hook(chunk, slot_begin, slot_end)
+//   pose_workspace      also sum the camera side of the gradient into this workspace (hg_raster_backward_pose)
 #include <torch/extension.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -24,7 +25,7 @@
 #include <tuple>
 #include <unordered_map>
 
-#include "../../include/hidegs_raster.h"
+#include "../../include/hidegs_geometry.h"
 
 namespace {
 
@@ -257,7 +258,8 @@ py::tuple rasterize_gaussians_backward(torch::Tensor background, torch::Tensor a
                                        torch::Tensor binningBuffer, torch::Tensor imageBuffer, bool render_geo, bool debug,
                                        c10::optional<torch::Tensor> sh_sink, double sh_beta,
                                        c10::optional<torch::Tensor> grad_arena, int64_t n_chunks, py::object chunk_hook,
-                                       c10::optional<torch::Tensor> sh_factor, bool skip_culled_rows) {
+                                       c10::optional<torch::Tensor> sh_factor, bool skip_culled_rows,
+                                       c10::optional<torch::Tensor> pose_workspace) {
   const auto dev = means3D.device();
   background = f32(background, "bg"); viewmatrix = f32(viewmatrix, "viewmatrix"); projmatrix = f32(projmatrix, "projmatrix");
   campos = f32(campos, "campos"); means3D = f32(means3D, "means3D"); colors = f32(colors, "colors_precomp");
@@ -343,10 +345,29 @@ py::tuple rasterize_gaussians_backward(torch::Tensor background, torch::Tensor a
       factor_ptr = sh_factor->data_ptr<float>();
       sink_used = true;  // the SH rows are not written: no dL_dsh is returned
     }
+    void* pose_ptr = nullptr;
+    if (pose_workspace.has_value() && pose_workspace->defined()) {
+      TORCH_CHECK(pose_workspace->is_contiguous() && pose_workspace->device() == dev &&
+                      pose_workspace->nbytes() >= hg_camera_pose_workspace_bytes(fullP),
+                  "pose_workspace must be a contiguous tensor of at least hg_camera_pose_workspace_bytes(N) bytes on ", dev);
+      pose_ptr = pose_workspace->data_ptr();
+    }
     const bool hooked = !chunk_hook.is_none() && n_chunks > 0 && !prezero;
     ChunkCtx cctx{hooked ? chunk_hook : py::none(), nullptr};
     int rc;
-    if (sink_ptr || factor_ptr || hooked || skip_culled_rows) {
+    if (pose_ptr) {
+      rc = hg_raster_backward_pose(
+          &in, (int32_t)R, ptr<int32_t>(radii), reinterpret_cast<const char*>(geomBuffer.data_ptr()),
+          reinterpret_cast<const char*>(binningBuffer.data_ptr()), reinterpret_cast<const char*>(imageBuffer.data_ptr()),
+          ptr<float>(all_map_pixels), ptr<float>(dL_dout_color), ptr<float>(dL_dout_all_map),
+          ptr<float>(dL_dout_plane_depth), has_depth_grad ? ptr<float>(dL_dout_invdepth) : nullptr, accum,
+          mptr<float>(dL_dmeans2D), nullptr, mptr<float>(dL_dopacity), mptr<float>(dL_dcolors),
+          has_depth_grad ? mptr<float>(dL_dinvdepths) : nullptr, mptr<float>(dL_dmeans3D), mptr<float>(dL_dcov3D),
+          mptr<float>(dL_dsh), mptr<float>(dL_dscales), mptr<float>(dL_drotations), mptr<float>(dL_dall_map),
+          hooked ? (int32_t)n_chunks : 1, hooked ? on_chunk : nullptr, &cctx, sink_ptr, (float)sh_beta, factor_ptr,
+          skip_culled_rows ? HG_BWD_SKIP_CULLED_ROWS : 0, pose_ptr, stream);
+      if (cctx.error) std::rethrow_exception(cctx.error);
+    } else if (sink_ptr || factor_ptr || hooked || skip_culled_rows) {
       rc = hg_raster_backward_chunked(
           &in, (int32_t)R, ptr<int32_t>(radii), reinterpret_cast<const char*>(geomBuffer.data_ptr()),
           reinterpret_cast<const char*>(binningBuffer.data_ptr()), reinterpret_cast<const char*>(imageBuffer.data_ptr()),
@@ -413,7 +434,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         py::arg("dL_dout_plane_depth"), py::arg("dL_dout_invdepth"), py::arg("sh"), py::arg("degree"), py::arg("campos"),
         py::arg("geomBuffer"), py::arg("R"), py::arg("binningBuffer"), py::arg("imageBuffer"), py::arg("render_geo"),
         py::arg("debug"), py::arg("sh_sink") = py::none(), py::arg("sh_beta") = 0.0, py::arg("grad_arena") = py::none(),
-        py::arg("n_chunks") = 0, py::arg("chunk_hook") = py::none(), py::arg("sh_factor") = py::none(), py::arg("skip_culled_rows") = false);
+        py::arg("n_chunks") = 0, py::arg("chunk_hook") = py::none(), py::arg("sh_factor") = py::none(), py::arg("skip_culled_rows") = false,
+        py::arg("pose_workspace") = py::none());
   m.def("mark_visible", &mark_visible);
   m.def("sh_sink_supported", &sh_sink_supported, py::arg("sh"), py::arg("indices") = py::none(),
         py::arg("parent_indices") = py::none());

@@ -25,7 +25,7 @@ sh_sink_supported = _hgC.sh_sink_supported
 
 
 def rasterize_gaussians_backward(*args, sh_sink=None, grad_arena=None, chunk_hook=None, sh_factor=None,
-                                 skip_culled_rows=False):
+                                 skip_culled_rows=False, pose_workspace=None):
     """RasterizeGaussiansBackwardCUDA (rasterize_points.cu:149-279), positional arguments as in the reference.
 
     Per-call extensions (keyword only; nothing is remembered between calls):
@@ -41,9 +41,11 @@ def rasterize_gaussians_backward(*args, sh_sink=None, grad_arena=None, chunk_hoo
                  at the view direction) followed by the camera centre; dL_dsh is returned as None
                  (parallel.FactoredExchange ships these 12 bytes per Gaussian instead of 192)
       skip_culled_rows  the gradient rows of culled Gaussians (radii <= 0) are left UNWRITTEN instead of zero-filled:
-                 only for a consumer that masks by `radii` (the trainer's fused prologue backward)."""
+                 only for a consumer that masks by `radii` (the trainer's fused prologue backward)
+      pose_workspace  tensor of >= hg_camera_pose_workspace_bytes(N) bytes: the call also sums the camera side of the
+                 gradient there (hg_raster_backward_pose; the camera pose refinement of the training step)."""
     sink, beta = sh_sink if sh_sink is not None else (None, 0.0)
     n_chunks, fn = chunk_hook if chunk_hook is not None else (0, None)
     return _hgC.rasterize_gaussians_backward(*args, sh_sink=sink, sh_beta=float(beta), grad_arena=grad_arena,
                                              n_chunks=int(n_chunks), chunk_hook=fn, sh_factor=sh_factor,
-                                             skip_culled_rows=bool(skip_culled_rows))
+                                             skip_culled_rows=bool(skip_culled_rows), pose_workspace=pose_workspace)

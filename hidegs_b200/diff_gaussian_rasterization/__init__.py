@@ -79,7 +79,8 @@ class _RasterizeGaussians(torch.autograd.Function):
         (grad_means2D, grad_colors_precomp, grad_opacities, grad_means3D, grad_cov3Ds_precomp, grad_sh, grad_scales,
          grad_rotations, grad_all_map) = _C.rasterize_gaussians_backward(
             *args, sh_sink=ctx.sh_sink() if ctx.sh_sink is not None else None, grad_arena=ctx.grad_arena,
-            sh_factor=ctx.sh_factor, skip_culled_rows=getattr(ctx, "skip_culled_rows", False))
+            sh_factor=ctx.sh_factor, skip_culled_rows=getattr(ctx, "skip_culled_rows", False),
+            pose_workspace=getattr(ctx, "pose_workspace", None))
         return (grad_means3D, grad_means2D, grad_sh, grad_colors_precomp, grad_opacities, grad_scales,
                 grad_rotations, grad_cov3Ds_precomp, grad_all_map, None)
 

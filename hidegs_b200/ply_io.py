@@ -211,6 +211,33 @@ def load_exposures(path, device="cuda"):
     return {name: torch.tensor(exposures[name], dtype=torch.float32, device=device) for name in exposures}
 
 
+def save_camera_poses(path, table, image_names, w2c=None):
+    """camera_poses.json of the per-image pose corrections (DESIGN.md §3 "Camera pose refinement"):
+    {image_name: {"xi": [rho 3, phi 3], "w2c": corrected 4x4 world-to-camera matrix (column convention)}}; `table` is the
+    [n, 8] table, `w2c` an optional {image_name: 4x4} (images without one get no "w2c")."""
+    rows = table.detach().double().cpu().numpy()
+    data = {}
+    for i, name in enumerate(image_names):
+        data[name] = {"xi": rows[i, :6].tolist()}
+        if w2c is not None and name in w2c:
+            data[name]["w2c"] = np.asarray(w2c[name], dtype=np.float64).reshape(4, 4).tolist()
+    with open(path, "w") as f:
+        json.dump(data, f, indent=2)
+
+
+def load_camera_poses(path):
+    """camera_poses.json -> {image_name: xi (6 floats)}, the `poses` argument of GaussianParams.setup_camera_poses."""
+    with open(path, "r") as f:
+        data = json.load(f)
+    out = {}
+    for name, entry in data.items():
+        xi = [float(x) for x in entry["xi"]]
+        if len(xi) != 6:
+            raise ValueError("camera_poses.json: %r has %d numbers in xi, expected 6" % (name, len(xi)))
+        out[name] = xi
+    return out
+
+
 def load_depth_params(path):
     """depth_params.json of graphdeco 3DGS's dataset readers: {image_name: {"scale", "offset"}} as a dict whose entries
     also carry "med_scale", the median of the POSITIVE scales of the file (0 when there are none).  DESIGN.md §3 "Depth

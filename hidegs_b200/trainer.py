@@ -81,6 +81,11 @@ class OptimizationParams:
     # graphdeco 3DGS's arguments/__init__.py values as recalled, not checked against a reference tree
     depth_l1_weight_init = 1.0
     depth_l1_weight_final = 0.01
+    # camera pose refinement (ViewShardedTrainer(train_poses=True)): Adam with eps 1e-8 over the whole [n, 8] table at
+    # constant rates, the translation one multiplied by spatial_lr_scale as position_lr_init is.  Nothing upstream
+    # defines these: they are this build's choice (translation in scene units, rotation in radians, per step)
+    pose_lr_translation = 0.0001
+    pose_lr_rotation = 0.0001
 
 
 class _ActivateParams(torch.autograd.Function):
@@ -245,6 +250,8 @@ class GaussianParams:
         self._sink_used = False
         self.exposure_mapping = None  # per-image exposure: setup_exposures
         self._exposure = self.exposure_grad = None
+        self.camera_pose_mapping = None  # per-image camera pose correction: setup_camera_poses
+        self._camera_pose = self.camera_pose_grad = None
 
     def setup_exposures(self, image_names, exposures=None):
         """Per-image exposure table of the reference's GaussianModel (`_exposure`, `exposure_mapping`; applied by
@@ -287,6 +294,79 @@ class GaussianParams:
         from . import ply_io
         names = sorted(self.exposure_mapping, key=self.exposure_mapping.get)
         ply_io.save_exposures(path, self._exposure, names)
+
+    def setup_camera_poses(self, image_names, poses=None):
+        """Per-image camera pose corrections (DESIGN.md §3 "Camera pose refinement"): row i of the leaf `_camera_pose`
+        [n, 8] is xi = (rho 3, phi 3, 2 zero pads) of image_names[i], applied in the camera frame (p_cam' = Exp(phi)
+        p_cam + rho); zero to start with, or poses[name] (a ply_io.load_camera_poses dict, which must cover every name).
+        Its `.grad` aliases `camera_pose_grad`.  The table is per image, not per Gaussian: densify_and_prune and resize
+        leave it alone."""
+        from . import camera_pose as cp
+        names = list(image_names)
+        if len(set(names)) != len(names):
+            raise ValueError("setup_camera_poses: duplicate image names")
+        table = torch.zeros((len(names), cp.ROW), dtype=torch.float32)
+        if poses is not None:
+            missing = [n for n in names if n not in poses]
+            if missing:
+                raise ValueError("setup_camera_poses: no pose for %s" % missing[:5])
+            for i, n in enumerate(names):
+                xi = torch.as_tensor(poses[n], dtype=torch.float32).cpu().reshape(-1)
+                if xi.numel() != 6:
+                    raise ValueError("setup_camera_poses: the pose of %r has %d numbers, expected 6" % (n, xi.numel()))
+                table[i, :6] = xi
+        self.camera_pose_mapping = {n: i for i, n in enumerate(names)}
+        self._camera_pose = table.to(self.param_arena.device).requires_grad_(True)
+        self.camera_pose_grad = torch.zeros_like(self._camera_pose, requires_grad=False)
+        self._camera_pose.grad = self.camera_pose_grad
+
+    def camera_pose_index(self, image_name):
+        """Row of `image_name` in the camera pose table; ValueError if there is no table or no such image."""
+        if self.camera_pose_mapping is None:
+            raise ValueError("no camera pose table: call setup_camera_poses(image_names) first")
+        try:
+            return self.camera_pose_mapping[image_name]
+        except KeyError:
+            raise ValueError("no camera pose for image %r" % (image_name,)) from None
+
+    def _corrected_matrices(self, k, viewmatrix, projmatrix, campos):
+        """[36] device buffer: viewmatrix' | projmatrix' | campos' | 0 of row k (hg_camera_pose_apply, no host read)."""
+        dev = self.param_arena.device
+        out = torch.empty(36, dtype=torch.float32, device=dev)
+        vm, pm, cp_ = (t.to(device=dev, dtype=torch.float32).contiguous() for t in (viewmatrix, projmatrix, campos))
+        with torch.cuda.device(dev):
+            rc = _G().hg_camera_pose_apply(vm.data_ptr(), pm.data_ptr(), cp_.data_ptr(), self._camera_pose.data_ptr(),
+                                           self._camera_pose.size(0), k, out.data_ptr(),
+                                           torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "camera_pose_apply")
+        return out
+
+    def corrected_camera(self, cam):
+        """A shallow copy of `cam` whose world_view_transform / full_proj_transform / camera_center (CUDA tensors) carry
+        the correction of its image, for render() and evaluation; intrinsics and image size are the camera's."""
+        import copy
+        if not self.fused:
+            raise ValueError("corrected_camera needs CUDA parameters")
+        buf = self._corrected_matrices(self.camera_pose_index(cam.image_name), cam.world_view_transform,
+                                       cam.full_proj_transform, cam.camera_center)
+        out = copy.copy(cam)
+        out.world_view_transform = buf[:16].view(4, 4)
+        out.full_proj_transform = buf[16:32].view(4, 4)
+        out.camera_center = buf[32:35]
+        return out
+
+    def save_camera_poses(self, path, cameras):
+        """camera_poses.json (ply_io.save_camera_poses): xi of every image of the table, and the corrected
+        world-to-camera matrix of those among `cameras` (float64 on the host, camera_pose.corrected_w2c)."""
+        from . import camera_pose as cp
+        from . import ply_io
+        names = sorted(self.camera_pose_mapping, key=self.camera_pose_mapping.get)
+        table = self._camera_pose.detach().double().cpu().numpy()
+        w2c = {}
+        for cam in cameras:
+            k = self.camera_pose_index(cam.image_name)
+            w2c[cam.image_name] = cp.corrected_w2c(cam.world_view_transform.detach().double().cpu().numpy(), table[k, :6])
+        ply_io.save_camera_poses(path, self._camera_pose, names, w2c)
 
     def _attach(self, param_arena, N):
         """Adopt `param_arena` (arena_layout(N)) with a fresh gradient arena of the same layout, the leaves and their
@@ -385,6 +465,7 @@ class ArenaAdam:
         self.exp_avg_sq = torch.zeros_like(params.param_arena)
         self.lr = dict(xyz=opt.position_lr_init * spatial_lr_scale, features=opt.feature_lr, opacity=opt.opacity_lr,
                        scaling=opt.scaling_lr, rotation=opt.rotation_lr)
+        self.spatial_lr_scale = spatial_lr_scale
         self.eps, self.step_count = eps, 0
 
     def resize(self, exp_avg, exp_avg_sq):
@@ -471,10 +552,11 @@ def balance_views(costs, world, speeds=None):
 class ViewShardedTrainer:
     train_exposure = False  # (class defaults: also read by trainers assembled without __init__)
     depth_regularization = False
+    train_poses = False
 
     def __init__(self, params: GaussianParams, background, opt=OptimizationParams, pipe=PipelineParams, group=None,
                  sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0, densify=False,
-                 scene_extent=None, train_exposure=False, depth_regularization=False):
+                 scene_extent=None, train_exposure=False, depth_regularization=False, train_poses=False):
         """`densify`: run the adaptive density control schedule of the OptimizationParams densify_* fields inside
         `step()` (off by default); it needs `scene_extent` (`cameras_extent(cameras)`) and turns the densification
         statistics on.
@@ -486,10 +568,29 @@ class ViewShardedTrainer:
         cam.depth_mask|, to the loss of every view whose camera carries a reliable prior (ply_io.attach_depth_prior;
         DESIGN.md §3 "Depth regularisation"), with w(it) the schedule of the OptimizationParams depth_l1_weight_*
         fields (off by default).  A view without a reliable prior, or a step with w(it) = 0, runs as it does with the
-        flag off."""
+        flag off.
+        `train_poses`: render every view through the pose correction of its `cam.image_name` and learn the table (off
+        by default; DESIGN.md §3 "Camera pose refinement"); it needs `params.setup_camera_poses(image_names)` first and
+        the direct executor (not HG_TRAINER_DIRECT=0: the autograd path has no camera gradient).  Every step zeroes the
+        pose gradient table, sums it over the ranks and steps it with its own Adam (eps 1e-8, dense over the whole
+        table, the constant rates OptimizationParams.pose_lr_translation x spatial_lr_scale and pose_lr_rotation)."""
+        import os
         self.params, self.bg, self.opt, self.pipe, self.group = params, background, opt, pipe, group
         if densify and scene_extent is None:
             raise ValueError("densify=True needs scene_extent (cameras_extent(cameras))")
+        self.train_poses = bool(train_poses)
+        if self.train_poses:
+            if params._camera_pose is None:
+                raise ValueError("train_poses=True needs params.setup_camera_poses(image_names)")
+            if not params.fused:
+                raise ValueError("train_poses=True needs CUDA parameters")
+            if os.environ.get("HG_TRAINER_DIRECT", "1") == "0":
+                raise ValueError("train_poses=True needs the direct executor: the autograd path (HG_TRAINER_DIRECT=0) "
+                                 "forms no camera gradient")
+            self.pose_exp_avg = torch.zeros_like(params._camera_pose, requires_grad=False)
+            self.pose_exp_avg_sq = torch.zeros_like(params._camera_pose, requires_grad=False)
+            self.pose_step_count = 0
+            self._pose_ws = None
         self.train_exposure = bool(train_exposure)
         if self.train_exposure:
             if params._exposure is None:
@@ -527,7 +628,6 @@ class ViewShardedTrainer:
         # frequency_regularization_pyramid_scale(iteration, warmup_iterations=1000) does; `start_iteration` resumes a run
         self.iteration = int(start_iteration)
         # autograd-free executor of a view (view_step_direct); HG_TRAINER_DIRECT=0 keeps the autograd path
-        import os
         self.direct = params.fused and os.environ.get("HG_TRAINER_DIRECT", "1") != "0"
         self._one = None
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -597,13 +697,15 @@ class ViewShardedTrainer:
         (loss value tensor, dict with "visibility_filter" (mask), "radii", "means2D_grad" — defined on the rendered rows
         only: the rasterizer's backward does not write the rows of culled Gaussians here); with train_exposure also
         "render", the exposed, clamped image the losses saw; with the depth term on this view also "depth_l1", the
-        unweighted masked inverse-depth L1 (device scalar)."""
+        unweighted masked inverse-depth L1 (device scalar); with train_poses also "pose_grad", this view's contribution
+        (dL/drho, dL/dphi) to its camera's row of the pose gradient table (device, 6 floats)."""
         o, p, T = self.opt, self.params, self._Tape
         dev = p.param_arena.device
         depth = self._depth_term(cam, iteration)  # (mono, mask, w) or None: the view runs as with the flag off
         exp_off = None  # byte offset of this camera's exposure row in the table / its gradient table
         if self.train_exposure:
             exp_off = 48 * p.exposure_index(cam.image_name)
+        pose_k = p.camera_pose_index(cam.image_name) if self.train_poses else None
         with torch.no_grad():
             # ---- forward
             # the activated parameters are the same for every view of one optimiser step: step() keeps them
@@ -617,6 +719,11 @@ class ViewShardedTrainer:
             e_i = torch.empty(0, dtype=torch.int32, device=dev)
             e_f = torch.empty(0, dtype=torch.float32, device=dev)
             rs = gr._raster_settings(cam, p, self.pipe, self.bg, 1.0, True, True, e_i, e_i, e_f, e_i)
+            pose_ws = None
+            if pose_k is not None:  # the corrected camera, formed on the device: every kernel below reads it
+                cbuf = p._corrected_matrices(pose_k, rs.viewmatrix, rs.projmatrix, rs.campos)
+                rs = rs._replace(viewmatrix=cbuf[:16].view(4, 4), projmatrix=cbuf[16:32].view(4, 4), campos=cbuf[32:35])
+                pose_ws = self._pose_workspace(p.N, dev)
             tM = T(True, False, True, False, False)
             all_map_in = gr._AllMap.forward(tM, xyz, scaling, rotation, rs.viewmatrix, rs.campos)
             if p.sh_sink:
@@ -717,14 +824,26 @@ class ViewShardedTrainer:
             # sink the SH gradient comes back as a dense tensor that the prologue backward adds to the arena row for
             # row, so every row of it (culled Gaussians, inactive SH bands) must be written
             tR.skip_culled_rows = tR.sh_sink is not None
+            tR.pose_workspace = pose_ws  # (None: the plain backward)
             (g_xyz, g_means2D, g_sh, _gc, g_op, g_sc, g_rot, _gcov, g_all_map_in, _n) = _RasterizeGaussians.backward(
                 tR, g_color, None, None, g_am, g_pd, g_inv)
             # all_map backward + scale-regulariser gradient + activation chain rule + accumulation into the arena: one
             # kernel over the rendered rows (hg_prologue_backward)
             self._prologue_backward(p, radii, rs, g_xyz, g_sh, g_op, g_sc, g_rot, g_all_map_in,
-                                    tSc.grad if tSc is not None else None, tT.partials[2] if tSc is not None else None)
+                                    tSc.grad if tSc is not None else None, tT.partials[2] if tSc is not None else None,
+                                    pose_ws)
+            pose_grad = None
+            if pose_k is not None:  # both partial sets -> dL/dxi of this view, added onto the camera's gradient row
+                pose_grad = torch.empty(6, dtype=torch.float32, device=dev)
+                with torch.cuda.device(dev):
+                    rc = _G().hg_camera_pose_grad_finish(
+                        p._camera_pose.data_ptr(), p._camera_pose.size(0), pose_k, p.N, pose_ws.data_ptr(),
+                        p.camera_pose_grad.data_ptr(), pose_grad.data_ptr(), torch.cuda.current_stream().cuda_stream)
+                _lib.check(rc, "camera_pose_grad_finish")
         out = {"visibility_filter": visible, "radii": radii, "means2D_grad": g_means2D,
                "num_rendered": int(tR.num_rendered)}
+        if pose_grad is not None:
+            out["pose_grad"] = pose_grad
         if exp_off is not None:
             out["render"] = image
         if depth_l1 is not None:
@@ -732,9 +851,11 @@ class ViewShardedTrainer:
         return loss, out
 
     @staticmethod
-    def _prologue_backward(p, radii, rs, g_xyz, g_feat, g_op, g_sc, g_rot, g_all_map, g_sc_extra, extra_scale):
+    def _prologue_backward(p, radii, rs, g_xyz, g_feat, g_op, g_sc, g_rot, g_all_map, g_sc_extra, extra_scale,
+                           pose_ws=None):
         """Gradients w.r.t. the activated parameters (+ dL/dall_map, + the scale regulariser's gradient) -> the raw
-        parameters' rows of the gradient arena, dst = beta * dst + grad, rows with radii <= 0 skipped."""
+        parameters' rows of the gradient arena, dst = beta * dst + grad, rows with radii <= 0 skipped.  `pose_ws`: also
+        sum the camera side of the all_map gradient there (hg_prologue_backward_pose)."""
         N = p.N
         if g_feat is not None and p._sink_used:  # (features also used outside the rasterizer: on top of the sink)
             p.grad_arena[p.slices["features"]].add_(g_feat.reshape(-1))
@@ -743,14 +864,17 @@ class ViewShardedTrainer:
             g_feat = torch.zeros((N, 16, 3), dtype=torch.float32, device=p.param_arena.device)
         ptr = lambda t: t.contiguous().data_ptr() if t is not None else None  # noqa: E731
         d = {k: p.grad_arena[p.slices[k]] for k in ("xyz", "features", "opacity", "scaling", "rotation")}
-        with torch.cuda.device(p.param_arena.device):
-            rc = _G().hg_prologue_backward(
-                p._scaling.data_ptr(), p._rotation.data_ptr(), p._opacity.data_ptr(), p._xyz.data_ptr(), N, 48,
+        args = (p._scaling.data_ptr(), p._rotation.data_ptr(), p._opacity.data_ptr(), p._xyz.data_ptr(), N, 48,
                 radii.data_ptr(), rs.viewmatrix.contiguous().data_ptr(), rs.campos.contiguous().data_ptr(),
                 ptr(g_xyz), ptr(g_feat), ptr(g_op), ptr(g_sc), ptr(g_rot), ptr(g_all_map), ptr(g_sc_extra),
                 ptr(extra_scale), 1.0 if p._grad_dirty else 0.0, d["xyz"].data_ptr(), d["features"].data_ptr(),
-                d["opacity"].data_ptr(), d["scaling"].data_ptr(), d["rotation"].data_ptr(),
-                torch.cuda.current_stream().cuda_stream)
+                d["opacity"].data_ptr(), d["scaling"].data_ptr(), d["rotation"].data_ptr())
+        with torch.cuda.device(p.param_arena.device):
+            st = torch.cuda.current_stream().cuda_stream
+            if pose_ws is None:
+                rc = _G().hg_prologue_backward(*args, st)
+            else:
+                rc = _G().hg_prologue_backward_pose(*args, pose_ws.data_ptr(), st)
         _lib.check(rc, "prologue_backward")
         p._grad_dirty = True
         p._sink_used = False
@@ -774,6 +898,9 @@ class ViewShardedTrainer:
         if self.depth_regularization:
             for view in views:  # a prior the step cannot use raises before the step has changed anything
                 self._depth_prior(view[0])
+        if self.train_poses:
+            for view in views:  # an image without a pose raises before the step has changed anything
+                self.params.camera_pose_index(view[0].image_name)
         self.iteration += 1
         timing = getattr(self, "timing", None)  # optional list: (start, views done, step done) CUDA events per step
         if timing is not None:
@@ -784,6 +911,10 @@ class ViewShardedTrainer:
             p = self.params
             p.exposure_grad.zero_()  # (n x 48 bytes; the views add their sums into it)
             p._exposure.grad = p.exposure_grad
+        if self.train_poses:
+            p = self.params
+            p.camera_pose_grad.zero_()  # (n x 32 bytes; the views add their gradients into it)
+            p._camera_pose.grad = p.camera_pose_grad
         total = None
         self.last_view_costs = []
         # optional (`self.time_views = True`): one CUDA event per view boundary, read back by last_view_ms()
@@ -830,6 +961,8 @@ class ViewShardedTrainer:
                 dist.all_reduce(self.visible, op=dist.ReduceOp.MAX, group=self.group)
             if self.train_exposure:
                 dist.all_reduce(self.params.exposure_grad, op=dist.ReduceOp.SUM, group=self.group)
+            if self.train_poses:
+                dist.all_reduce(self.params.camera_pose_grad, op=dist.ReduceOp.SUM, group=self.group)
             if total_views is not None:
                 n_views = total_views
             else:  # ranks may hold uneven shards of views[rank::world]: count what was really rendered
@@ -839,6 +972,8 @@ class ViewShardedTrainer:
         self.adam.step(grad_scale=1.0 / max(n_views, 1), visible_mask=self.visible if self.sparse_adam else None)
         if self.train_exposure:
             self._exposure_adam_step(1.0 / max(n_views, 1))
+        if self.train_poses:
+            self._pose_adam_step(1.0 / max(n_views, 1))
         if getattr(self, "densify", False):
             self._density_schedule()
         if timing is not None:
@@ -909,6 +1044,31 @@ class ViewShardedTrainer:
                                    self.exposure_exp_avg_sq.data_ptr(), n, 12, None, None, 0,
                                    float(self.exposure_lr(self.iteration)), 0.9, 0.999, 1e-8, self.exposure_step_count,
                                    float(grad_scale), 0, 0.0, torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "adam_step")
+
+    def _pose_workspace(self, N, dev):
+        """Partial sums of the pose variants of the backward (hg_camera_pose_workspace_bytes(N)), grown with N; every
+        byte the finish reads is written by the view's two kernels first."""
+        need = int(_G().hg_camera_pose_workspace_bytes(N))
+        if self._pose_ws is None or self._pose_ws.numel() < need:
+            self._pose_ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        return self._pose_ws
+
+    @torch.no_grad()
+    def _pose_adam_step(self, grad_scale):
+        """Adam over the whole pose table (torch.optim.Adam semantics, eps 1e-8, its own step count, the gradient
+        scaled by 1 / views as the Gaussians' is): rho (the 3 head columns) at pose_lr_translation x spatial_lr_scale,
+        phi at pose_lr_rotation; the pad columns have zero gradient and stay zero.  One launch."""
+        p = self.params
+        if self.pose_exp_avg.shape != p._camera_pose.shape:
+            raise RuntimeError("the camera pose table was replaced after the trainer was built (setup_camera_poses)")
+        self.pose_step_count += 1
+        lr_t = float(self.opt.pose_lr_translation) * float(getattr(self.adam, "spatial_lr_scale", 1.0))
+        with torch.cuda.device(p.param_arena.device):
+            rc = _G().hg_adam_step(p._camera_pose.data_ptr(), p.camera_pose_grad.data_ptr(), self.pose_exp_avg.data_ptr(),
+                                   self.pose_exp_avg_sq.data_ptr(), p._camera_pose.size(0), p._camera_pose.size(1), None,
+                                   None, 0, float(self.opt.pose_lr_rotation), 0.9, 0.999, 1e-8, self.pose_step_count,
+                                   float(grad_scale), 3, lr_t, torch.cuda.current_stream().cuda_stream)
         _lib.check(rc, "adam_step")
 
     def _zero_densification_stats(self):

@@ -84,6 +84,32 @@ HG_API int hg_prologue_backward(const float *raw_scaling, const float *raw_rotat
                                 float beta, float *d_xyz, float *d_features, float *d_opacity, float *d_scaling,
                                 float *d_rotation, void *stream);
 
+/* Per-image camera pose refinement (DESIGN.md §3 "Camera pose refinement").  A pose table is [n_poses, 8] fp32 on the
+ * device: row k = xi_k = (rho 3, phi 3, 2 zero pads), applied in the camera frame, p_cam' = Exp(phi) p_cam + rho.
+ *   hg_camera_pose_apply: out [36] = viewmatrix' [16] | projmatrix' [16] | campos' [3] | 0 of the camera corrected by
+ *     row `index` (host int; the table is not read on the host): viewmatrix' = viewmatrix C^T, projmatrix' =
+ *     viewmatrix' times the camera's intrinsic projection, campos' its centre.  A zero row gives the input bit for bit.
+ *   hg_camera_pose_workspace_bytes(N): the partial sums of the pose variants of the backward for N Gaussians (0 for
+ *     N <= 0 or N > INT32_MAX).
+ *   hg_prologue_backward_pose: hg_prologue_backward that also sums the camera side of the all_map gradient, one row per
+ *     256-row CTA, into its part of `pose_workspace` (the same workspace as hg_raster_backward_pose's).
+ *   hg_camera_pose_grad_finish: sums both parts in double in a fixed order (the bits depend on N only, not on the SM
+ *     count) and ADDS dL/dxi = (g, J_l(phi)^T (tau - rho x g)) onto row `index` of pose_grad_table [n_poses, 8]; with
+ *     view_grad6 != NULL those 6 floats are also written there. */
+HG_API int hg_camera_pose_apply(const float *viewmatrix, const float *projmatrix, const float *campos,
+                                const float *pose_table, int32_t n_poses, int32_t index, float *out, void *stream);
+HG_API size_t hg_camera_pose_workspace_bytes(int64_t N);
+HG_API int hg_prologue_backward_pose(const float *raw_scaling, const float *raw_rotation, const float *raw_opacity,
+                                     const float *xyz, int64_t N, int32_t F, const int32_t *radii,
+                                     const float *viewmatrix, const float *campos, const float *g_xyz,
+                                     const float *g_features, const float *g_opacity, const float *g_scaling,
+                                     const float *g_rotation, const float *g_all_map, const float *g_scaling_extra,
+                                     const float *extra_scale, float beta, float *d_xyz, float *d_features,
+                                     float *d_opacity, float *d_scaling, float *d_rotation, void *pose_workspace,
+                                     void *stream);
+HG_API int hg_camera_pose_grad_finish(const float *pose_table, int32_t n_poses, int32_t index, int64_t N,
+                                      const void *workspace, float *pose_grad_table, float *view_grad6, void *stream);
+
 /* Camera intrinsics as Camera.get_calib_matrix_nerf builds them (scene/cameras.py:93-96,135-138). */
 typedef struct hg_intrinsics {
   float fx, fy, cx, cy;

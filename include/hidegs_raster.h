@@ -223,6 +223,26 @@ HG_API int hg_raster_backward_chunked(const hg_raster_inputs *in, int32_t R,
                                        void *chunk_ctx, float *sh_sink, float sh_beta, float *sh_factor,
                                        int32_t flags, void *stream);
 
+/* hg_raster_backward_chunked that also forms the camera side of the gradient, for per-image camera pose refinement
+ * (DESIGN.md §3 "Camera pose refinement"; viewmatrix / projmatrix / campos are the view's CORRECTED camera, e.g. the
+ * output of hg_camera_pose_apply, include/hidegs_geometry.h).  Every rendered slot sums dL/dp_cam over every path and
+ * its torque; each 128-slot CTA of the per-Gaussian part writes the sum of its slots (double, fixed order) to its row
+ * of `pose_workspace` (hg_camera_pose_workspace_bytes(N) bytes, 16-byte aligned; rows are indexed by the global CTA,
+ * so n_chunks does not change a bit).  hg_prologue_backward_pose adds the all_map part and hg_camera_pose_grad_finish
+ * turns both into the camera's gradient row.  Needs every Gaussian as one slot: render / parent indices and P != N are
+ * rejected.  Every other argument as in hg_raster_backward_chunked. */
+HG_API int hg_raster_backward_pose(const hg_raster_inputs *in, int32_t R,
+                       const int32_t *radii,
+                       const char *geom_buffer, const char *binning_buffer,
+                       const char *image_buffer,
+                       const float *all_map_pixels, const float *dL_dpix, const float *dL_dout_all_map,
+                       const float *dL_dout_plane_depth, const float *dL_dout_invdepth,
+                       char *accum, float *dL_dmeans2D, float *dL_dconic, float *dL_dopacity,
+                       float *dL_dcolors, float *dL_dinvdepths, float *dL_dmeans3D, float *dL_dcov3D,
+                       float *dL_dsh, float *dL_dscales, float *dL_drotations, float *dL_dall_map,
+                       int32_t n_chunks, hg_chunk_fn on_chunk, void *chunk_ctx, float *sh_sink, float sh_beta,
+                       float *sh_factor, int32_t flags, void *pose_workspace, void *stream);
+
 /* Test / diagnostic accessor.  The library never materialises the reference's 64-bit tile|depth keys: it buckets the
  * tile instances by tile (counts from the preprocess pass, one scan, one scatter) and sorts every tile's list by
  * (depth, slot) in shared memory -- same final order as the reference's global 45..47-bit sort, one pass over the
