@@ -9,7 +9,8 @@ EXPORTED_SYMBOLS = (
     "hg_interpolation_weights", "hg_hier_interpolate", "hg_hier_interpolate_backward",
     "hg_dist2_knn3_workspace_bytes", "hg_dist2_knn3", "hg_densify_workspace_bytes", "hg_densify_plan", "hg_densify_apply",
     "hg_reset_opacity", "hg_camera_pose_apply", "hg_camera_pose_workspace_bytes", "hg_prologue_backward_pose",
-    "hg_camera_pose_grad_finish",
+    "hg_camera_pose_grad_finish", "hg_mcmc_workspace_bytes", "hg_mcmc_regularizer", "hg_mcmc_inject_noise",
+    "hg_mcmc_relocate", "hg_mcmc_grow",
 )
 
 
@@ -58,6 +59,11 @@ def lib():
         "hg_prologue_backward_pose": (ci, [vp, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f32, vp,
                                            vp, vp, vp, vp, vp, vp]),
         "hg_camera_pose_grad_finish": (ci, [vp, i32, i32, i64, vp, vp, vp, vp]),
+        "hg_mcmc_workspace_bytes": (sz, [i64]),
+        "hg_mcmc_regularizer": (ci, [vp, vp, p64, i64, i32, f64, f64, f64, f64, vp, vp, vp, vp]),
+        "hg_mcmc_inject_noise": (ci, [vp, p64, i64, i32, f64, vp, ctypes.c_uint64, vp]),
+        "hg_mcmc_relocate": (ci, [vp, vp, vp, p64, i64, i32, f64, vp, i64, ctypes.c_uint64, vp, vp, vp]),
+        "hg_mcmc_grow": (ci, [vp, vp, vp, p64, i64, vp, vp, vp, p64, i64, i32, f64, vp, ctypes.c_uint64, vp, vp]),
     }
     for name, (res, args) in proto.items():
         fn = getattr(L, name)

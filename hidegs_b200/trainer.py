@@ -86,6 +86,23 @@ class OptimizationParams:
     # defines these: they are this build's choice (translation in scene units, rotation in radians, per step)
     pose_lr_translation = 0.0001
     pose_lr_rotation = 0.0001
+    # 3DGS-MCMC densification (ViewShardedTrainer(mcmc=True); DESIGN.md §3 "MCMC densification"): refine (relocate,
+    # then grow) every mcmc_refine_interval steps in (mcmc_refine_from_iter, mcmc_refine_until_iter), position noise
+    # every step.  The 3DGS-MCMC paper's and gsplat MCMCStrategy's values as recalled, not checked against a reference
+    mcmc_refine_from_iter = 500
+    mcmc_refine_until_iter = 25_000
+    mcmc_refine_interval = 100
+    mcmc_min_opacity = 0.005
+    mcmc_grow_factor = 1.05
+    mcmc_noise_lr = 5e5
+    mcmc_opacity_reg = 0.01
+    mcmc_scale_reg = 0.01
+    # the position learning-rate schedule of graphdeco 3DGS (xyz_scheduler_args), used in MCMC mode only:
+    # get_expon_lr_func(position_lr_init * s, position_lr_final * s, lr_delay_mult=position_lr_delay_mult,
+    # max_steps=position_lr_max_steps), s = spatial_lr_scale.  Without MCMC the xyz rate stays position_lr_init * s
+    position_lr_final = 0.0000016
+    position_lr_delay_mult = 0.01
+    position_lr_max_steps = 30_000
 
 
 class _ActivateParams(torch.autograd.Function):
@@ -216,6 +233,117 @@ def densify_arenas(param_arena, exp_avg, exp_avg_sq, N, accum, max_grad, min_opa
                                 int(seed) & 0xFFFFFFFFFFFFFFFF, ws.data_ptr(), st)
     _lib.check(rc, "densify_apply")
     return new[0], new[1], new[2], counts
+
+
+# ---- 3DGS-MCMC densification (DESIGN.md §3 "MCMC densification"; include/hidegs_geometry.h hg_mcmc_*) ------------------
+def mcmc_refines(it, opt):
+    """Whether step `it` refines (relocate, then grow) after its optimiser update: refine_from < it < refine_until and
+    it a multiple of refine_interval."""
+    return opt.mcmc_refine_from_iter < it < opt.mcmc_refine_until_iter and it % opt.mcmc_refine_interval == 0
+
+
+def mcmc_grow_target(N, cap_max, grow_factor):
+    """Row count after a growth of N rows: min(cap_max, int(grow_factor * N)); N itself when that is not larger."""
+    return max(N, min(int(cap_max), int(grow_factor * N)))
+
+
+def mcmc_workspace(N, dev):
+    """A zero-filled workspace of the hg_mcmc_* entries for N rows (the regulariser's counter starts at zero)."""
+    return torch.zeros(int(_G().hg_mcmc_workspace_bytes(N)), dtype=torch.uint8, device=dev)
+
+
+def _offsets(N):
+    starts, _total = arena_layout(N)
+    return (ctypes.c_int64 * 5)(*[starts[n] for n, _ in GROUPS])
+
+
+def _sources(sources, n, N, dev):
+    """Injected draws as int64 device rows in [0, N) (checked on the host: a test path, it may synchronise)."""
+    s = torch.as_tensor(sources).to(device=dev, dtype=torch.int64).contiguous().view(-1)
+    if n is not None and s.numel() != n:
+        raise ValueError("sources must hold %d rows, got %d" % (n, s.numel()))
+    if s.numel() and (int(s.min()) < 0 or int(s.max()) >= N):
+        raise ValueError("sources must be rows in [0, %d)" % N)
+    return s
+
+
+def mcmc_regularizer(param_arena, grad_arena, N, opacity_reg, scale_reg, grad_mult=1.0, loss_mult=0.0, loss=None,
+                     workspace=None, skybox_points=0):
+    """Reg = opacity_reg mean(o) + scale_reg mean(s) over the N rows: adds grad_mult dReg into the opacity and scaling
+    rows of `grad_arena`, adds loss_mult Reg onto the device scalar `loss` (may be None) and returns Reg as a device
+    scalar (None, and no launch, when both weights are 0).  `workspace`: mcmc_workspace(N) (allocated when None)."""
+    if opacity_reg == 0.0 and scale_reg == 0.0:
+        return None
+    dev = param_arena.device
+    ws = mcmc_workspace(N, dev) if workspace is None else workspace
+    value = torch.empty((), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        rc = _G().hg_mcmc_regularizer(param_arena.data_ptr(), grad_arena.data_ptr(), _offsets(N), N, int(skybox_points),
+                                      float(opacity_reg), float(scale_reg), float(grad_mult), float(loss_mult),
+                                      value.data_ptr(), loss.data_ptr() if loss is not None else None, ws.data_ptr(),
+                                      torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "mcmc_regularizer")
+    return value
+
+
+def mcmc_inject_noise(param_arena, N, scale, seed=0, normals=None, skybox_points=0):
+    """gsplat's inject_noise_to_position in place: xyz += scale sigma(100 ((1 - o) - 0.995)) (R diag(s^2) R^T) z with
+    scale = lr_xyz(it) * noise_lr; z from Philox4x32-10 keyed by `seed`, or `normals` [N, 3]."""
+    dev = param_arena.device
+    if normals is not None:
+        normals = normals.to(device=dev, dtype=torch.float32).contiguous()
+        if tuple(normals.shape) != (N, 3):
+            raise ValueError("normals must be [%d, 3], got %s" % (N, tuple(normals.shape)))
+    with torch.cuda.device(dev):
+        rc = _G().hg_mcmc_inject_noise(param_arena.data_ptr(), _offsets(N), N, int(skybox_points), float(scale),
+                                       normals.data_ptr() if normals is not None else None,
+                                       int(seed) & 0xFFFFFFFFFFFFFFFF, torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "mcmc_inject_noise")
+
+
+def mcmc_relocate_arenas(param_arena, exp_avg, exp_avg_sq, N, min_opacity=0.005, seed=0, sources=None,
+                         skybox_points=0, workspace=None):
+    """Relocate the dead rows (o <= min_opacity) of N-row arenas onto live ones drawn with probability o, in place
+    (DESIGN.md §3 "MCMC densification").  Returns (param_arena, exp_avg, exp_avg_sq, counts) with counts =
+    dict(dead=, alive=) as int64 device scalars: nothing is read back.  Draws from Philox4x32-10 keyed by `seed`, or
+    `sources` (the source row of each dead row in row order; checked on the host)."""
+    dev = param_arena.device
+    ws = mcmc_workspace(N, dev) if workspace is None else workspace
+    src = _sources(sources, None, N, dev) if sources is not None else None
+    out = torch.empty(2, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        rc = _G().hg_mcmc_relocate(param_arena.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), _offsets(N), N,
+                                   int(skybox_points), float(min_opacity),
+                                   src.data_ptr() if src is not None and src.numel() else None,
+                                   src.numel() if src is not None else 0, int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                   out.data_ptr(), ws.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "mcmc_relocate")
+    return param_arena, exp_avg, exp_avg_sq, dict(dead=out[0], alive=out[1])
+
+
+def mcmc_grow_arenas(param_arena, exp_avg, exp_avg_sq, N, n_target, min_opacity=0.005, seed=0, sources=None,
+                     skybox_points=0, workspace=None):
+    """Grow N-row arenas to `n_target` rows (N < n_target <= 2 N): n_target - N draws over all rows with probability
+    o (Philox4x32-10 keyed by `seed`, or `sources` [n_target - N]); the drawn rows take (o', s') and zero moments, and
+    their copies are appended in draw order with zero moments.  Returns (new parameter arena, new exp_avg, new
+    exp_avg_sq, counts = dict(added=, n=)) with host ints; n_target <= N returns the arenas unchanged."""
+    n_target = int(n_target)
+    if n_target <= N:
+        return param_arena, exp_avg, exp_avg_sq, dict(added=0, n=N)
+    if n_target > 2 * N:
+        raise ValueError("mcmc_grow_arenas: n_target %d exceeds 2 N = %d" % (n_target, 2 * N))
+    dev = param_arena.device
+    ws = mcmc_workspace(N, dev) if workspace is None else workspace
+    src = _sources(sources, n_target - N, N, dev) if sources is not None else None
+    _starts, total = arena_layout(n_target)
+    new = [torch.empty(total, dtype=torch.float32, device=dev) for _ in range(3)]  # every float written by the kernels
+    with torch.cuda.device(dev):
+        rc = _G().hg_mcmc_grow(param_arena.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), _offsets(N), N,
+                               new[0].data_ptr(), new[1].data_ptr(), new[2].data_ptr(), _offsets(n_target), n_target,
+                               int(skybox_points), float(min_opacity), src.data_ptr() if src is not None else None,
+                               int(seed) & 0xFFFFFFFFFFFFFFFF, ws.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "mcmc_grow")
+    return new[0], new[1], new[2], dict(added=n_target - N, n=n_target)
 
 
 def cameras_extent(cameras):
@@ -553,10 +681,12 @@ class ViewShardedTrainer:
     train_exposure = False  # (class defaults: also read by trainers assembled without __init__)
     depth_regularization = False
     train_poses = False
+    mcmc = False
 
     def __init__(self, params: GaussianParams, background, opt=OptimizationParams, pipe=PipelineParams, group=None,
                  sparse_adam=True, densification_stats=False, cache_ground_truth=False, start_iteration=0, densify=False,
-                 scene_extent=None, train_exposure=False, depth_regularization=False, train_poses=False):
+                 scene_extent=None, train_exposure=False, depth_regularization=False, train_poses=False, mcmc=False,
+                 mcmc_cap_max=None):
         """`densify`: run the adaptive density control schedule of the OptimizationParams densify_* fields inside
         `step()` (off by default); it needs `scene_extent` (`cameras_extent(cameras)`) and turns the densification
         statistics on.
@@ -573,8 +703,26 @@ class ViewShardedTrainer:
         by default; DESIGN.md §3 "Camera pose refinement"); it needs `params.setup_camera_poses(image_names)` first and
         the direct executor (not HG_TRAINER_DIRECT=0: the autograd path has no camera gradient).  Every step zeroes the
         pose gradient table, sums it over the ranks and steps it with its own Adam (eps 1e-8, dense over the whole
-        table, the constant rates OptimizationParams.pose_lr_translation x spatial_lr_scale and pose_lr_rotation)."""
+        table, the constant rates OptimizationParams.pose_lr_translation x spatial_lr_scale and pose_lr_rotation).
+        `mcmc`: 3DGS-MCMC densification instead of adaptive density control (off by default; DESIGN.md §3 "MCMC
+        densification"): the opacity / scale regulariser in every step, relocation of dead Gaussians and growth by
+        mcmc_grow_factor up to `mcmc_cap_max` Gaussians on the schedule of the OptimizationParams mcmc_* fields, position
+        noise after every optimiser update, and graphdeco's position learning-rate schedule.  It needs CUDA parameters
+        without skybox points and mcmc_cap_max >= params.N, and excludes `densify`.  The model's size never exceeds
+        mcmc_cap_max; nothing of it reads back to the host, and every rank computes the same bits (the arenas are
+        identical after the exchange and the Adam step, and every kernel is deterministic in its inputs and seed)."""
         import os
+        if mcmc:  # (refusals before anything changes)
+            if densify:
+                raise ValueError("mcmc=True and densify=True are two densification strategies: choose one")
+            if params.skybox_points:
+                raise ValueError("mcmc=True: models with skybox points are not supported")
+            if mcmc_cap_max is None or int(mcmc_cap_max) < params.N:
+                raise ValueError("mcmc=True needs mcmc_cap_max >= params.N = %d, got %r" % (params.N, mcmc_cap_max))
+            if not 1.0 <= float(opt.mcmc_grow_factor) <= 2.0:
+                raise ValueError("mcmc_grow_factor must be in [1, 2], got %r" % (opt.mcmc_grow_factor,))
+            if not params.fused:
+                raise ValueError("mcmc=True needs CUDA parameters")
         self.params, self.bg, self.opt, self.pipe, self.group = params, background, opt, pipe, group
         if densify and scene_extent is None:
             raise ValueError("densify=True needs scene_extent (cameras_extent(cameras))")
@@ -613,6 +761,15 @@ class ViewShardedTrainer:
         self.densify, self.scene_extent = densify, scene_extent
         densification_stats = densification_stats or densify
         self.adam = ArenaAdam(params, opt)
+        self.mcmc = bool(mcmc)
+        if self.mcmc:
+            from .optim import get_expon_lr_func
+            sc = self.adam.spatial_lr_scale
+            self.mcmc_cap_max = int(mcmc_cap_max)
+            self.xyz_lr = get_expon_lr_func(opt.position_lr_init * sc, opt.position_lr_final * sc,
+                                            lr_delay_mult=opt.position_lr_delay_mult,
+                                            max_steps=opt.position_lr_max_steps)
+            self._mcmc_ws = mcmc_workspace(params.N, params.param_arena.device)
         # the reference steps its optimiser on the rows that were visible (`optimizer.step(relevant)`, OurAdam.py:106)
         self.sparse_adam = sparse_adam and params.param_arena.is_cuda
         self.visible = torch.zeros(params.N, dtype=torch.uint8, device=params.param_arena.device)
@@ -969,6 +1126,14 @@ class ViewShardedTrainer:
                 cnt = torch.tensor([float(n_views)], device=self.params.grad_arena.device)
                 dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=self.group)
                 n_views = int(round(float(cnt.item())))
+        if self.mcmc:  # the same arena on every rank after the exchange: the regulariser adds the same bits everywhere
+            p, o = self.params, self.opt
+            self.adam.lr["xyz"] = float(self.xyz_lr(self.iteration))
+            if total is None:
+                total = torch.zeros((), dtype=torch.float32, device=p.param_arena.device)
+            mcmc_regularizer(p.param_arena, p.grad_arena, p.N, o.mcmc_opacity_reg, o.mcmc_scale_reg,
+                             grad_mult=float(max(n_views, 1)), loss_mult=float(len(views)), loss=total,
+                             workspace=self._mcmc_ws)
         self.adam.step(grad_scale=1.0 / max(n_views, 1), visible_mask=self.visible if self.sparse_adam else None)
         if self.train_exposure:
             self._exposure_adam_step(1.0 / max(n_views, 1))
@@ -976,6 +1141,8 @@ class ViewShardedTrainer:
             self._pose_adam_step(1.0 / max(n_views, 1))
         if getattr(self, "densify", False):
             self._density_schedule()
+        if self.mcmc:
+            self._mcmc_schedule()
         if timing is not None:
             ev[2].record()
             timing.append(ev)
@@ -1128,6 +1295,64 @@ class ViewShardedTrainer:
                                    20 if it > o.opacity_reset_interval else None)
         if it % o.opacity_reset_interval == 0:
             self.reset_opacity()
+
+    def _require_mcmc(self, what):
+        if not self.mcmc:
+            raise RuntimeError("%s needs ViewShardedTrainer(mcmc=True, mcmc_cap_max=...)" % what)
+
+    @torch.no_grad()
+    def relocate_dead(self, seed=None):
+        """3DGS-MCMC relocation in place: every dead Gaussian (opacity <= mcmc_min_opacity) becomes a copy of a live one
+        drawn with probability proportional to its opacity, and the sources' opacity and scale are corrected (DESIGN.md
+        §3 "MCMC densification").  The moments of sources and destinations are zeroed.  `seed` keys the draws (default:
+        the iteration).  Returns dict(dead=, alive=) as int64 device scalars: nothing is read back."""
+        self._require_mcmc("relocate_dead")
+        p = self.params
+        counts = mcmc_relocate_arenas(p.param_arena, self.adam.exp_avg, self.adam.exp_avg_sq, p.N,
+                                      self.opt.mcmc_min_opacity, self.iteration if seed is None else seed,
+                                      skybox_points=p.skybox_points, workspace=self._mcmc_ws)[3]
+        p._act = None
+        self._step_activations = None
+        return counts
+
+    @torch.no_grad()
+    def grow(self, seed=None):
+        """3DGS-MCMC growth: N' = min(mcmc_cap_max, int(mcmc_grow_factor N)) Gaussians, the new ones copies of rows drawn
+        with probability proportional to opacity (sources and copies share the corrected opacity and scale; their
+        moments start at zero).  Goes through GaussianParams.resize / ArenaAdam.resize, which re-create the gradient
+        exchange (collectively across ranks); the visibility mask and the densification statistics start afresh.
+        `seed` keys the draws (default: the iteration).  Returns dict(added=, n=) with host ints computed from N alone:
+        nothing is read back.  At the cap nothing changes."""
+        self._require_mcmc("grow")
+        p = self.params
+        n_target = mcmc_grow_target(p.N, self.mcmc_cap_max, self.opt.mcmc_grow_factor)
+        if n_target <= p.N:
+            return dict(added=0, n=p.N)
+        new_p, new_m, new_v, counts = mcmc_grow_arenas(
+            p.param_arena, self.adam.exp_avg, self.adam.exp_avg_sq, p.N, n_target, self.opt.mcmc_min_opacity,
+            self.iteration if seed is None else seed, skybox_points=p.skybox_points, workspace=self._mcmc_ws)
+        p.resize(new_p, counts["n"])
+        self.adam.resize(new_m, new_v)
+        self.visible = torch.zeros(p.N, dtype=torch.uint8, device=new_p.device)
+        if self.densification_stats:
+            self._zero_densification_stats()
+        self._mcmc_ws = mcmc_workspace(p.N, new_p.device)
+        self._step_activations = None
+        return counts
+
+    @torch.no_grad()
+    def _mcmc_schedule(self):
+        """gsplat MCMCStrategy.step_post_backward after the optimiser step of step `it`: relocate then grow when
+        mcmc_refines(it), then position noise at lr_xyz(it) * mcmc_noise_lr on every step (past the refinement window
+        too), keyed by the iteration."""
+        it = self.iteration
+        if mcmc_refines(it, self.opt):
+            self.relocate_dead()
+            self.grow()
+        p = self.params
+        mcmc_inject_noise(p.param_arena, p.N, self.adam.lr["xyz"] * self.opt.mcmc_noise_lr, seed=it,
+                          skybox_points=p.skybox_points)
+        p._act = None
 
     def _add_densification_stats(self, pkg):
         g = pkg["means2D_grad"] if "means2D_grad" in pkg else pkg["viewspace_points"].grad

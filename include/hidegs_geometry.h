@@ -187,6 +187,42 @@ HG_API int hg_densify_apply(const float *old_param, const float *old_exp_avg, co
                             uint64_t seed, const void *workspace, void *stream);
 HG_API int hg_reset_opacity(float *opacity, float *exp_avg, float *exp_avg_sq, int64_t N, void *stream);
 
+/* 3DGS-MCMC densification over the training arenas (DESIGN.md §3 "MCMC densification"; gsplat's MCMCStrategy).
+ * Arenas and group_offsets as for hg_densify_plan; o = sigmoid(opacity), s = exp(scaling), R = build_rotation(q) with
+ * hg_densify_apply's bits.  No entry reads anything back to the host; a model with skybox_points != 0 is rejected.
+ *   hg_mcmc_workspace_bytes(N): the workspace of every entry below for N rows.  Zero-fill it once before its first
+ *     use: the regulariser's ticket counter lives there and every call leaves it at zero again; the sampling buffers
+ *     (written before they are read) never overlap it, so one workspace serves the regulariser and the refinements.
+ *   hg_mcmc_regularizer: Reg = opacity_reg mean_i o_i + scale_reg mean_{i,a} s_ia over the N rows.  ADDS grad_mult
+ *     dReg into the opacity and scaling rows of `grad` (an arena of the same layout); writes Reg to `value` and adds
+ *     loss_mult Reg onto `loss_inout` (device floats, each may be NULL).  The sums are per-CTA doubles added by the
+ *     last CTA in a fixed order: the bits depend on N only, not on the SM count.  No launch when both weights are 0.
+ *   hg_mcmc_inject_noise: xyz += scale sigma(100 ((1 - o) - 0.995)) (R diag(s^2) R^T) z, z ~ N(0, I) from
+ *     Philox4x32-10 (key = seed, counter = (row, 2)) or z = normals [N, 3] when non-NULL.  scale = lr_xyz(it) noise_lr.
+ *   hg_mcmc_relocate (in place): rows with !(o > (float)min_opacity) are dead.  Draw j < n_dead picks a live row with
+ *     probability o / sum(o): u from Philox4x32-10 (key = seed, counter = (j, 0), 53 bits), the smallest i with
+ *     cdf[i] > u cdf[N-1] over the double prefix sum of the live weights; or sources[j] (j < n_sources, int64 device
+ *     rows; other slots draw nothing) when non-NULL.  Every row drawn c times takes (o', s') of the relocation formula
+ *     with n = min(c + 1, 51), and dead row j (in row order) becomes a copy of its source; the moments of sources and
+ *     destinations are zeroed.  out_counts (device int64 [2], may be NULL) receives (dead rows, live rows).  Nothing
+ *     changes when no row is dead or none is alive.
+ *   hg_mcmc_grow: N < new_n <= 2 N.  Draws j < new_n - N over all rows weighted by o (counter = (j, 1)), or
+ *     sources [new_n - N] (int64 device rows in [0, N)); uniform over the rows when no row has a positive weight.  The new arenas hold the old rows, the drawn ones with (o', s')
+ *     and zero moments, followed by copies of the sources in draw order with zero moments; pad floats are zeroed. */
+HG_API size_t hg_mcmc_workspace_bytes(int64_t N);
+HG_API int hg_mcmc_regularizer(const float *param, float *grad, const int64_t *group_offsets, int64_t N,
+                               int32_t skybox_points, double opacity_reg, double scale_reg, double grad_mult,
+                               double loss_mult, float *value, float *loss_inout, void *workspace, void *stream);
+HG_API int hg_mcmc_inject_noise(float *param, const int64_t *group_offsets, int64_t N, int32_t skybox_points,
+                                double scale, const float *normals, uint64_t seed, void *stream);
+HG_API int hg_mcmc_relocate(float *param, float *exp_avg, float *exp_avg_sq, const int64_t *group_offsets, int64_t N,
+                            int32_t skybox_points, double min_opacity, const int64_t *sources, int64_t n_sources,
+                            uint64_t seed, int64_t *out_counts, void *workspace, void *stream);
+HG_API int hg_mcmc_grow(const float *old_param, const float *old_exp_avg, const float *old_exp_avg_sq,
+                        const int64_t *old_offsets, int64_t N, float *new_param, float *new_exp_avg,
+                        float *new_exp_avg_sq, const int64_t *new_offsets, int64_t new_n, int32_t skybox_points,
+                        double min_opacity, const int64_t *sources, uint64_t seed, void *workspace, void *stream);
+
 /* Hierarchy LOD cut (SURVEY.md §8(f) f1).  nodes [N,7] i32 (types.h:47-56: depth, parent, start, count_leafs,
  * count_merged, start_children, count_children), boxes [N,2,4] f32 (min xyz + extent, max xyz + pad), viewpoint [3] on
  * the device.  hg_expand_to_size = Switching::expandToSize (runtime_switching.cu:496-527): for every node whose
